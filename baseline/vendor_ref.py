@@ -1,10 +1,10 @@
 #!/usr/bin/env python
 """Copies the three files of the UNMODIFIED reference that the hot path needs into the git-ignored baseline/_ref/
-(BASELINE.md section 4.1), so that the reference itself can be timed -- and used as a second checker -- on the GPU
-box, which only receives /root/repo.  Nothing under baseline/_ref/ is tracked or imported by the product; only
-bench.py's CPU arm uses it, through ``import_reference()`` below.
+(BASELINE.md section 4.1), so that the reference itself can be timed -- and used as a second checker -- by
+bench.py's CPU arm.  Nothing under baseline/_ref/ is tracked or imported by the product; only bench.py's CPU arm
+uses it, through ``import_reference()`` below, and reports it unavailable when nothing was vendored.
 
-    python baseline/vendor_ref.py            # in the build container, where /root/reference exists
+    python baseline/vendor_ref.py <checkout of AnnaLew/pangenomix>/pangenomix
 """
 import os
 import shutil
@@ -12,18 +12,15 @@ import sys
 import types
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF_SRC = "/root/reference/pangenomix"
 REF_DST = os.path.join(HERE, "_ref", "pangenomix")
 FILES = ["__init__.py", "pangenome_analysis.py", "sparse_utils.py"]
 
 
-def vendor():
-    if not os.path.isdir(REF_SRC):
-        return False
+def vendor(src):
+    """Copies FILES from ``src``, the reference's package directory."""
     os.makedirs(REF_DST, exist_ok=True)
     for name in FILES:
-        shutil.copyfile(os.path.join(REF_SRC, name), os.path.join(REF_DST, name))
-    return True
+        shutil.copyfile(os.path.join(src, name), os.path.join(REF_DST, name))
 
 
 def available():
@@ -34,7 +31,7 @@ def import_reference():
     """(pangenome_analysis, sparse_utils) of the vendored reference.  statsmodels (imported at
     pangenome_analysis.py:18, used only at :380, off the hot path) is absent from the image and stubbed."""
     if not available():
-        raise ImportError("baseline/_ref is empty: run baseline/vendor_ref.py in the build container")
+        raise ImportError("baseline/_ref is empty: run baseline/vendor_ref.py <reference package directory>")
     import importlib.util
     for name in ("statsmodels", "statsmodels.stats"):
         sys.modules.setdefault(name, types.ModuleType(name))
@@ -65,4 +62,7 @@ def import_reference():
 
 
 if __name__ == "__main__":
-    print("vendored" if vendor() else "no /root/reference here; baseline/_ref %s" % ("present" if available() else "absent"))
+    if len(sys.argv) != 2:
+        sys.exit("usage: python baseline/vendor_ref.py <reference package directory>")
+    vendor(sys.argv[1])
+    print("vendored into %s" % REF_DST)

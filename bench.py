@@ -1,9 +1,14 @@
 #!/usr/bin/env python
 """bench.py -- pan/core permutations per second on B200 (BASELINE.json's metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c4|c2|c1|c5|c3] [--perms P]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c4|c2|c1|c5|c3] [--perms P] [--dump-outputs DIR]
     python bench.py --impl reference ...          # the CPU arm (oracle C port, all host threads)
     torchrun --nproc-per-node N ... bench.py --gpus N ...   # one rank per GPU
+
+The library is the one build() (python -m pangenomix_b200.build) left in the tree; bench.py compiles nothing.
+--dump-outputs DIR writes what the timed path returned in its last step as DIR/<name>.npy (float64, at most
+64 MB in all; rows of a larger output are a fixed seeded sample), so that two builds can be compared on the
+same inputs: the table, the permutations and the Bernoulli points are all drawn from fixed seeds.
 
 A step is one pass of the hot path over one batch of permutations: P genome orders
 (per GPU) -> P pan/core curves, through libpgx_b200 (include/pgx.h).  The default workload
@@ -74,7 +79,38 @@ def parse_args():
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"],
                     help="weak (default, what the driver runs): every GPU rarefies the config's permutation count; "
                          "strong: the config's permutations are split over the GPUs, as BASELINE.json words C4")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step to DIR/<name>.npy (rank 0)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_LIMIT = 64_000_000            # bytes --dump-outputs writes at most
+
+
+def dump_rows(n_rows, row_bytes, reserved):
+    """Row indices --dump-outputs keeps of an output of ``n_rows`` rows: all of them when they fit DUMP_LIMIT,
+    else a sample fixed by seed 0 (so two runs with the same arguments keep the same rows)."""
+    k = min(n_rows, (DUMP_LIMIT - reserved) // (row_bytes + 8))
+    if k == n_rows:
+        return np.arange(n_rows)
+    return np.sort(np.random.RandomState(0).choice(n_rows, k, replace=False))
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes every array of ``arrays`` (float32 or float64) as out_dir/<name>.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    total = 0
+    for name, arr in arrays.items():
+        arr = np.ascontiguousarray(arr)
+        assert arr.dtype in (np.float32, np.float64), (name, arr.dtype)
+        path = os.path.join(out_dir, name + ".npy")
+        np.save(path, arr)
+        total += os.path.getsize(path)
+    assert total <= DUMP_LIMIT, "dumped %d bytes" % total
+    log("[bench] wrote %s (%.1f MB) to %s" % (", ".join(sorted(arrays)), total / 1e6, out_dir))
 
 
 # --------------------------------------------------------------------------------------
@@ -164,8 +200,7 @@ def python_reference_sample(coo, eng=None, n_iter=1):
 def run_reference(args, rank, world):
     if rank != 0:
         return
-    from oracle import build as oracle_build, cport
-    oracle_build.build()
+    from oracle import cport
     from pangenomix_b200 import synth
     coo = load_matrix(args.workload, 0, lambda: None)
     perms_cfg = args.perms or synth.CONFIGS[args.workload][4]
@@ -175,8 +210,13 @@ def run_reference(args, rank, world):
         cport.curves_direct(gm, perms[:threads], n_threads=threads)
     t = time.perf_counter()
     for _ in range(args.steps):
-        cport.curves_direct(gm, perms, n_threads=threads)
+        pan, core = cport.curves_direct(gm, perms, n_threads=threads)
     dt = time.perf_counter() - t
+    if args.dump_outputs:
+        curves = np.hstack([pan, core])
+        rows = dump_rows(curves.shape[0], curves.shape[1] * 8, curves.shape[1] * 8 + 4096)
+        dump_outputs(args.dump_outputs, {"curves": curves[rows], "curve_rows": rows.astype(np.float64),
+                                         "mean_curve": curves.mean(axis=0)})
     value = perms.shape[0] * args.steps / dt
     sample = "%d permutations per step (of the config's %d), %d threads, oracle C port of " \
              "pangenome_analysis.py:81-90" % (perms.shape[0], perms_cfg, threads)
@@ -277,13 +317,10 @@ def run_b200(args, rank, world, local_rank):
     import torch
     import torch.distributed as dist
     from pangenomix_b200 import _native, engine, synth
-    from pangenomix_b200 import build as pgx_build
 
     assert torch.cuda.is_available(), "bench.py needs a CUDA device (no CPU fallback)"
     torch.cuda.set_device(local_rank)
     device = torch.device("cuda", local_rank)
-    if rank == 0:
-        pgx_build.build()
     if world > 1:
         dist.init_process_group("nccl", device_id=device)
 
@@ -393,6 +430,13 @@ def run_b200(args, rank, world, local_rank):
         torch.cuda.synchronize()
         elapsed = sum(a.elapsed_time(b) for a, b in brackets)
     w1 = time.perf_counter()
+    if args.dump_outputs and rank == 0:
+        # the curves of the last timed step, before the profile pass below overwrites the buffer
+        last = d_outs[(step_no[0] - 1) % n_buf][:perms_n]
+        rows = dump_rows(perms_n, 2 * n * 8, 2 * n * 8 + 4096)
+        sample = last.index_select(0, torch.from_numpy(rows).to(device)).double().cpu().numpy()
+        mean = (last.sum(dim=0, dtype=torch.int64).double() / perms_n).cpu().numpy()
+        dump_outputs(args.dump_outputs, {"curves": sample, "curve_rows": rows.astype(np.float64), "mean_curve": mean})
     barrier()
     ms = torch.tensor([elapsed], dtype=torch.float64, device=device)
     if world > 1:
@@ -616,8 +660,7 @@ def run_b200(args, rank, world, local_rank):
     })
     cpu = None
     if (world == 1 or args.cpu_check) and not args.no_cpu_baseline:
-        from oracle import build as oracle_build, cport
-        oracle_build.build()
+        from oracle import cport
         threads = os.cpu_count() or 1
         gm, sample_perms, t1 = cpu_sample(coo, n, args.cpu_seconds, threads)
         t0 = time.perf_counter()
@@ -788,10 +831,8 @@ def run_bernoulli(args):
     import torch
     import oracle
     from pangenomix_b200 import _native, engine, synth
-    from pangenomix_b200 import build as pgx_build
     assert torch.cuda.is_available(), "bench.py needs a CUDA device (no CPU fallback)"
     torch.cuda.set_device(0)
-    pgx_build.build()
     g, n = args.genes, 400
     x, _, _ = synth.bernoulli_grid_matrix(g, n, seed=3)
     grid = engine.BernoulliGrid(x, device="cuda:0")
@@ -814,7 +855,7 @@ def run_bernoulli(args):
     torch.cuda.synchronize()
     sampler = ClockSampler(0)
     time.sleep(0.2)
-    steps = max(args.steps, 200)
+    steps = args.steps
     launches0 = _native.launch_count()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     w0 = time.perf_counter()
@@ -824,6 +865,9 @@ def run_bernoulli(args):
     e1.record()
     torch.cuda.synchronize()
     w1 = time.perf_counter()
+    if args.dump_outputs:
+        res = grid._res.cpu().numpy()                 # [LL, gradient] at the point of the last step
+        dump_outputs(args.dump_outputs, {"loglikelihood": res[:1], "gradient": res[1:]})
     ms = e0.elapsed_time(e1)
     launches = _native.launch_count() - launches0
     clocks = sampler.window(w0, w1)
