@@ -361,6 +361,37 @@ int pgx_ks_montecarlo(const uint32_t *d_raw, int64_t iterations, int64_t n_sampl
 int pgx_ks_montecarlo_host(uint32_t *mt_key, int32_t *mt_pos, int64_t iterations, int64_t n_samples,
                            const double *h_choice_cdf, const double *h_model_cdf, int32_t sim_limit, double *h_ks_sim);
 
+/* Seeded genome orders generated on the device, for rarefaction curves whose statistics matter rather than numpy's
+ * particular shuffles (the drop-in pgx_estimate_pan_core keeps numpy's stream).  Permutation i (a 64-bit global
+ * index) is a pure function of (seed, i): results do not depend on block sizes, on how a range is split over calls
+ * or over GPUs.  The recipe (oracle/perm_np.py restates it in numpy):
+ *
+ *   Philox4x32-10 (Salmon et al., SC'11) with key (seed & 0xffffffff, seed >> 32); lo / hi = low / high 32 bits of i.
+ *   B(N) = the largest power of two <= ceil(N / 2), b = log2 B (B <= 16,384 for N <= 65,503).
+ *   1. Genome c draws bucket  w >> (32 - b)  (0 when b == 0), w = word c % 4 of Philox({c / 4, lo, hi, 0}).
+ *   2. Each bucket's genomes are put in ascending genome order.
+ *   3. Bucket k of m genomes is Fisher-Yates shuffled from the top: for j = m - 1 down to 1, draw v = w & mask(j)
+ *      (mask(j) = smallest 2^t - 1 >= j) until v <= j, then swap entries j and v.  The t-th word (t = 0, 1, ...)
+ *      bucket k consumes is word t % 4 of Philox({k, lo, hi, 0x80000000 | t / 4}).
+ *   4. The row is bucket 0, bucket 1, ..., bucket B - 1 concatenated.
+ * Every bucket is a uniformly random ordering of its members and the bucket draws do not depend on genome labels, so
+ * the distribution of the row is invariant under relabelling the genomes: it is exactly uniform for every B (with
+ * Philox taken as ideal), unlike sorting by random keys, whose ties make it only approximately so.
+ *   d_perms : [n_perm][N] uint16, rows first .. first + n_perm - 1 (the layout pgx_pan_core_curves takes), 2-byte
+ *             aligned.  1 <= N <= 65503, 0 <= first, 0 <= n_perm <= 2^31 - 1.
+ * One CTA per permutation, the row in shared memory.  Asynchronous on ``stream``. */
+int pgx_random_perms(uint64_t seed, int64_t first, int64_t n_perm, int32_t n_genomes, uint16_t *d_perms, void *stream);
+
+/* Exact column moments of a block of curves (int32 [n_rows][width], width even, 8-byte aligned):
+ *   d_sum[c] = sum of column c (int64), d_sumsq[c] = sum of squares (uint64), d_min[c] / d_max[c] (int32).
+ *   accumulate == 0 : the outputs are first set to 0, 0, INT32_MAX, INT32_MIN;  != 0 : the block is added to them.
+ * Integer accumulators make the result independent of the order of the atomics.  Exact while the rows accumulated
+ * into one set of outputs, n, satisfy  n * max|value|^2 < 2^63  (sums of squares then also fit an int64, which a
+ * caller combining several GPUs relies on); for pan/core curves max|value| <= G, the table's genes: at G = 2 M about
+ * 2.3 M permutations.  The caller enforces the bound.  Asynchronous on ``stream``. */
+int pgx_curve_moments(const int32_t *d_curves, int64_t n_rows, int64_t width, int64_t *d_sum, uint64_t *d_sumsq,
+                      int32_t *d_min, int32_t *d_max, int32_t accumulate, void *stream);
+
 #ifdef __cplusplus
 }
 #endif

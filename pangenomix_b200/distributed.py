@@ -9,6 +9,10 @@ NVLink on the B200 box; gloo in the CPU tests of this host-side logic).
 The only RNG that matters is rank 0's global numpy stream -- rank 0 draws all
 ``num_iter`` shuffles exactly as the reference does (pangenome_analysis.py:84-85) and
 broadcasts the table.
+
+``estimate_pan_core_summary_sharded`` needs neither: its genome orders come from the seeded
+on-device stream, which every rank evaluates for its own block of indices, and the ranks
+combine exact integer moments with one all-reduce.
 """
 from __future__ import annotations
 
@@ -136,6 +140,65 @@ def estimate_pan_core_size_sharded(df_genes, num_iter, log_batch=-1, group=None,
     pan_cols = ['Pan' + str(x) for x in range(1, num_strains + 1)]
     core_cols = ['Core' + str(x) for x in range(1, num_strains + 1)]
     return pd.DataFrame(curves.astype(np.float64), index=iter_index, columns=pan_cols + core_cols, copy=False)
+
+
+def estimate_pan_core_summary_sharded(df_genes, num_iter, seed=0, group=None, dst=None, compute=None, engine=None):
+    """Multi-GPU ``estimate_pan_core_summary``: the same DataFrame, bit for bit, for every world size, on the ranks
+    that receive it (all ranks for ``dst=None``), None elsewhere.
+
+    Rank r reduces the permutations ``shard_bounds(num_iter, world, r)`` of the seeded on-device stream to integer
+    moments on its own GPU; there is no broadcast of permutations and no gather of curves, only one all-reduce of
+    4 x 2N integers (SUM of the sums and of the sums of squares as int64 bit patterns, MIN / MAX of the extremes).
+    Every rank must call it with the same table, ``num_iter`` and ``seed``; numpy's RNG is not touched.
+
+    engine  : a PanCoreEngine on this rank's GPU (default: the engine cache of the single-GPU call).
+    compute : instead of an engine, callable(first, count) -> (sum int64, sumsq uint64, min int32, max int32) numpy
+              arrays of length 2N for permutations first .. first + count - 1 (the CPU tests of this host-side logic
+              inject one; tensors then live on the CPU).
+    """
+    import torch
+    from .engine import check_moment_bound, CurveMoments
+    from .pangenome_analysis import summary_frame
+    dist = _dist()
+    world, rank = dist.get_world_size(group), dist.get_rank(group)
+    num_iter = int(num_iter)
+    if num_iter < 1:
+        raise ValueError("num_iter must be at least 1")
+    n_genes, num_strains = df_genes.shape
+    check_moment_bound(num_iter, n_genes)
+    if compute is None and engine is None:
+        from .pangenome_analysis import _engine_for
+        engine = _engine_for(df_genes)
+    device = engine.device if engine is not None else torch.device("cpu")
+    lo, hi = shard_bounds(num_iter, world, rank)
+    width = 2 * num_strains
+
+    problem = None
+    try:
+        if engine is not None:
+            parts = list(engine.summary_device(hi - lo, seed, first=lo))
+        else:
+            parts = [torch.zeros(width, dtype=torch.int64), torch.zeros(width, dtype=torch.int64),
+                     torch.full((width,), 2 ** 31 - 1, dtype=torch.int32), torch.full((width,), -2 ** 31, dtype=torch.int32)]
+            if hi > lo:
+                local = compute(lo, hi - lo)
+                for k, (arr, dtype) in enumerate(zip(local, (np.int64, np.uint64, np.int32, np.int32))):
+                    arr = np.ascontiguousarray(arr, dtype=dtype)
+                    if arr.shape != (width,):
+                        raise ValueError("compute returned shape %s, expected (%d,)" % (arr.shape, width))
+                    parts[k] = torch.from_numpy(arr.view(np.int64) if dtype == np.uint64 else arr)
+    except Exception as exc:                                    # noqa: BLE001 - reported after the ranks agree
+        problem = exc
+    if not _agree(problem is None, device, group):
+        if problem is not None:
+            raise problem
+        raise RuntimeError("another rank failed to compute its share of the summary")
+    for tensor, op in zip(parts, (dist.ReduceOp.SUM, dist.ReduceOp.SUM, dist.ReduceOp.MIN, dist.ReduceOp.MAX)):
+        dist.all_reduce(tensor, op=op, group=group)
+    if dst is not None and rank != dst:
+        return None
+    s, q, mn, mx = (t.cpu().numpy() for t in parts)
+    return summary_frame(CurveMoments(num_iter, s, q.view(np.uint64), mn, mx), num_strains)
 
 
 class CurveGather:

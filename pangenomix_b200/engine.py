@@ -5,6 +5,7 @@ arithmetic happens in libpgx_b200.so (hand-written sm_100a kernels, include/pgx.
 """
 from __future__ import annotations
 
+import collections
 import ctypes
 import os
 
@@ -74,6 +75,54 @@ def draw_legacy_permutations(n, count, out=None):
     _native.check(_native.load().pgx_legacy_shuffles(
         key.ctypes.data, ctypes.byref(pos), n, count, out.ctypes.data))
     np.random.set_state((state[0], key, int(pos.value), state[3], state[4]))
+    return out
+
+
+MAX_SEED = 2 ** 64 - 1
+MOMENT_LIMIT = 2 ** 63        # n_perm * max|value|^2 must stay below this for pgx_curve_moments to be exact
+
+
+class CurveMoments(collections.namedtuple("CurveMoments", "n sum sumsq min max")):
+    """Exact column moments of ``n`` pan/core curves: sum (int64), sum of squares (uint64), min and max (int32),
+    each of length 2N (Pan1..PanN, Core1..CoreN)."""
+
+
+def check_moment_bound(n_perm, n_genes):
+    """Raises ValueError unless ``n_perm`` curves of a table of ``n_genes`` genes keep the integer moments exact."""
+    if int(n_perm) * max(int(n_genes), 1) ** 2 >= MOMENT_LIMIT:
+        raise ValueError("%d permutations of a table of %d genes overflow the exact int64 moments "
+                         "(n_perm * G^2 must stay below 2^63)" % (int(n_perm), int(n_genes)))
+
+
+def _check_stream_range(seed, first, n_perm):
+    seed, first, n_perm = int(seed), int(first), int(n_perm)
+    if not 0 <= seed <= MAX_SEED:
+        raise ValueError("seed must be in [0, 2^64)")
+    if first < 0 or n_perm < 0 or first + n_perm > 2 ** 63 - 1:
+        raise ValueError("permutation indices must lie in [0, 2^63 - 1)")
+    return seed, first, n_perm
+
+
+def random_permutations_device(n_genomes, n_perm, seed, first=0, device=None, out=None):
+    """Permutations ``first .. first + n_perm - 1`` of the seeded on-device stream (pgx_random_perms; the recipe is
+    in include/pgx.h) as a CUDA int16 tensor [n_perm, n_genomes] holding uint16 genome indices.
+
+    Permutation i depends on (seed, i) only, so any split of an index range over calls or GPUs gives the same rows.
+    Asynchronous on the current torch stream.
+    """
+    torch = _torch()
+    dev = _require_cuda(device)
+    seed, first, n_perm = _check_stream_range(seed, first, n_perm)
+    n_genomes = int(n_genomes)
+    if not 1 <= n_genomes <= 65503:
+        raise ValueError("n_genomes = %d outside 1 .. 65503" % n_genomes)
+    if out is None:
+        out = torch.empty((n_perm, n_genomes), dtype=torch.int16, device=dev)
+    elif out.shape != (n_perm, n_genomes) or out.element_size() != 2 or not out.is_contiguous() or out.device != dev:
+        raise ValueError("out must be a contiguous 16-bit [n_perm, n_genomes] tensor on %s" % dev)
+    with torch.cuda.device(dev):
+        _native.check(_native.load().pgx_random_perms(
+            seed, first, n_perm, n_genomes, out.data_ptr(), torch.cuda.current_stream(dev).cuda_stream))
     return out
 
 
@@ -216,6 +265,47 @@ class PanCoreEngine:
                 print('\tIteration', num_iter, 'of', num_iter)
         np.random.set_state((state[0], key, int(pos.value), state[3], state[4]))
         return out
+
+    # ---- seeded on-device rarefaction, reduced on the device ----------------------------
+    def summary_device(self, num_iter, seed, first=0, block=None):
+        """Exact column moments of the curves of permutations ``first .. first + num_iter - 1`` of the seeded
+        on-device stream, as CUDA tensors (sum int64, sum of squares int64 holding uint64 bits, min int32,
+        max int32; each [2N]).  Blocks of ``block`` permutations (default: about 1 GB of permutations and curves)
+        go through generate -> curves_device -> pgx_curve_moments, reusing one permutation and one curve buffer;
+        nothing crosses PCIe.  ``num_iter == 0`` gives sums 0, min INT32_MAX, max INT32_MIN.  Asynchronous on the
+        current torch stream."""
+        torch = _torch()
+        seed, first, num_iter = _check_stream_range(seed, first, num_iter)
+        check_moment_bound(num_iter, self.n_genes)
+        n = self.n_genomes
+        if block is None:
+            block = max(1, 10 ** 9 // (10 * n))              # 2N bytes of permutation + 8N bytes of curves each
+        block = max(1, min(int(block), num_iter))
+        dev = self.device
+        moments = (torch.empty(2 * n, dtype=torch.int64, device=dev), torch.empty(2 * n, dtype=torch.int64, device=dev),
+                   torch.empty(2 * n, dtype=torch.int32, device=dev), torch.empty(2 * n, dtype=torch.int32, device=dev))
+        ptrs = [m.data_ptr() for m in moments]
+        with torch.cuda.device(dev):
+            stream = torch.cuda.current_stream(dev).cuda_stream
+            if num_iter == 0:
+                _native.check(self.lib.pgx_curve_moments(None, 0, 2 * n, *ptrs, 0, stream))
+                return moments
+            perms = torch.empty((block, n), dtype=torch.int16, device=dev)
+            curves = torch.empty((block, 2 * n), dtype=torch.int32, device=dev)
+            done = 0
+            while done < num_iter:
+                k = min(block, num_iter - done)
+                random_permutations_device(n, k, seed, first + done, device=dev, out=perms[:k])
+                self.curves_device(perms[:k], out=curves[:k])
+                _native.check(self.lib.pgx_curve_moments(curves.data_ptr(), k, 2 * n, *ptrs, 1 if done else 0, stream))
+                done += k
+        return moments
+
+    def summary(self, num_iter, seed, first=0, block=None):
+        """summary_device() brought to the host as a CurveMoments of numpy arrays (waits for the device)."""
+        s, q, lo, hi = self.summary_device(num_iter, seed, first=first, block=block)
+        return CurveMoments(int(num_iter), s.cpu().numpy(), q.cpu().numpy().view(np.uint64), lo.cpu().numpy(),
+                            hi.cpu().numpy())
 
 
 def fit_heaps_device(curves, n_points=None):

@@ -12,6 +12,9 @@ reference; the work is done by libpgx_b200 on a B200:
   counted on the GPU, scipy Nelder-Mead / Shapiro-Wilk on the host as in the reference, and the Monte-Carlo KS
   simulation on the GPU (pgx_ks_montecarlo_host), consuming the global numpy RNG exactly as ``np.random.choice`` does
 
+Extension beside the drop-in: ``estimate_pan_core_summary`` -- mean / std / min / max of the pan/core curves over
+genome orders drawn on the GPU from a seeded counter-based stream (not numpy's), reduced on the GPU.
+
 Not provided (out of scope, SURVEY.md section 2): the coordinate-descent variant the
 reference marks "DON'T USE THIS" and the mlst wrapper.
 """
@@ -156,6 +159,58 @@ def estimate_pan_core_size(df_genes, num_iter, log_batch=-1, device=None):
     # (pandas 3 copies by default)
     return pd.DataFrame(curves, index=_labels(('Iter',), num_iter),
                         columns=_labels(('Pan', 'Core'), num_strains), copy=False)
+
+
+def estimate_pan_core_summary(df_genes, num_iter, seed=0, device=None):
+    '''
+    Mean, spread and range of the pan/core curves over ``num_iter`` random genome orders, computed without
+    building the (num_iter, 2N) table: genome orders are drawn on the GPU from a seeded counter-based stream
+    (pgx_random_perms; permutation i is a function of (seed, i) alone), rarefied there and reduced there to exact
+    integer moments.  Only 4 x 2N numbers come back to the host.
+
+    Unlike estimate_pan_core_size() this does not replay numpy's shuffles: it leaves ``np.random`` untouched and
+    the orders it uses are not the reference's.  It prints nothing.
+
+    Parameters
+    ----------
+    df_genes : LightSparseDataFrame
+        Sparse binary gene x genome table (anything with .shape and a scipy .data)
+    num_iter : int
+        Number of random genome orders (>= 1)
+    seed : int
+        Seed of the stream, 0 <= seed < 2^64
+    device : optional CUDA device (default: current device)
+
+    Returns
+    -------
+    df_stats : pd.DataFrame
+        float64, index ['mean', 'std', 'min', 'max'], columns Pan1..PanN, Core1..CoreN.  ``mean`` equals
+        plot.calculate_mean() of the full table of the same orders bit for bit; ``std`` has ddof=1 as pandas
+        (NaN for num_iter == 1, exactly 0 where every order gives the same value).  ``df_stats.loc[['mean']]``
+        can be passed to fit_heaps_by_iteration() / fit_heaps_by_iteration_gpu().
+    '''
+    num_iter = int(num_iter)
+    if num_iter < 1:
+        raise ValueError("num_iter must be at least 1")
+    _, num_strains = df_genes.shape
+    engine = _engine_for(df_genes, device)
+    return summary_frame(engine.summary(num_iter, seed), num_strains)
+
+
+def summary_frame(moments, num_strains):
+    """The DataFrame of estimate_pan_core_summary() from exact integer moments (engine.CurveMoments)."""
+    n = int(moments.n)
+    total = np.asarray(moments.sum, dtype=np.int64)
+    mean = total.astype(np.float64) / n                     # sums below 2^53 convert exactly: pandas' mean
+    if n > 1:
+        # n * sum(x^2) - sum(x)^2 in Python integers, divided once: the correctly rounded ddof=1 variance
+        num = np.asarray(moments.sumsq, dtype=np.uint64).astype(object) * n - total.astype(object) ** 2
+        std = np.sqrt(np.array(num / (n * (n - 1)), dtype=np.float64))
+    else:
+        std = np.full(total.shape, np.nan)
+    data = np.vstack([mean, std, np.asarray(moments.min, dtype=np.float64), np.asarray(moments.max, dtype=np.float64)])
+    return pd.DataFrame(data, index=['mean', 'std', 'min', 'max'], columns=_labels(('Pan', 'Core'), num_strains),
+                        copy=False)
 
 
 def compute_bernoulli_grid_core_genome(df_genes_dense,
