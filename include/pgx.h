@@ -36,7 +36,7 @@
 extern "C" {
 #endif
 
-#define PGX_VERSION 320
+#define PGX_VERSION 321
 
 enum {
     PGX_OK = 0,
@@ -46,7 +46,7 @@ enum {
 };
 
 /* Device-resident plan of a BINARY gene x genome presence/absence table, built once per
- * matrix by pgx_plan_create (below; pangenomix_b200/plan.py is its numpy specification) from
+ * matrix by pgx_plan_create (below; oracle/plan_np.py is its numpy specification) from
  * ``df_genes.data`` -- the same object estimate_pan_core_size reads at pangenome_analysis.py:74.
  * Genes fall into three groups:
  *
@@ -232,55 +232,6 @@ size_t pgx_heaps_scratch_bytes(int64_t n_points);
 int pgx_heaps_fit(const void *d_curves, int32_t is_f64, int64_t n_curves, int64_t n_points, int64_t stride,
                   double *d_fit, int32_t *d_info, void *d_scratch, void *stream);
 
-/* Host-side helper of the planner (no GPU work): orders the entries of the list rows so that the lanes
- * of a shared-memory wavefront of the list kernel hit distinct banks (pangenomix_b200/plan.py,
- * _bank_ordered_chunks; the layout is the one struct pgx_plan documents).
- *   flat / ptr        : sorted folded lists of the n_rows list rows, concatenated (int32) / offsets (int64)
- *   block_*           : per sub-block of 32 rows: first chunk, chunks per row, first row, rows (int64 [n_blocks])
- *   modulus           : lanes per 128-byte wavefront: 8, 16 or 32 (= 64 / perms_per_cta, capped)
- *   colour_max_chunks : rows of more chunks use the cheap positional order instead of the edge colouring
- *   chunks            : out, uint16 [sum(block_nch) * 32 * 8]
- *   n_threads         : host threads (0 = choose) */
-int pgx_plan_bank_order(const int32_t *flat, const int64_t *ptr, int64_t n_rows,
-                        const int64_t *block_first, const int64_t *block_nch,
-                        const int64_t *block_first_row, const int64_t *block_rows, int64_t n_blocks,
-                        int32_t n_genomes, int32_t modulus, int32_t colour_max_chunks,
-                        uint16_t *chunks, int32_t n_threads);
-
-/* Host-side helper of the planner: the bit-sliced bitmap d_bits of struct pgx_plan for the long rows
- * ``long_gene`` (gene ids, in superblock order) of a gene-major CSR (indptr int64, indices int32).
- * ``bits`` (uint32 [n_superblocks * n_genomes * 32 * slice_words]) must be zero-initialised. */
-int pgx_plan_build_bitmap(const int64_t *indptr, const int32_t *indices, const int64_t *long_gene,
-                          int64_t n_long, int32_t n_genomes, int32_t slice_words, uint32_t *bits,
-                          int32_t n_threads);
-
-/* Host-side helpers of the planner for the table ingest (no GPU work; threaded; n_threads 0 = choose).
- * They do what pangenome_analysis.py:74-75 asks of scipy (``df_genes.data`` COO -> compressed rows), gene-major.
- *
- * pgx_plan_coo_to_csr: COO entries (row = gene, col = genome; every stored value 1 -- the caller checks) ->
- *   canonical CSR: indptr int64 [n_genes + 1], indices int32 [nnz] ascending inside a row, colsum int32
- *   [n_genomes].  Duplicate (gene, genome) pairs are kept and counted in *n_duplicates (scipy's tocsr would
- *   sum them to 2, a non-binary table: the caller rejects it).
- * pgx_plan_folded_lists: for list row r (gene genes[r]) the ascending list of its present genomes
- *   (use_abs[r] == 0) or absent genomes (use_abs[r] != 0) into flat[ptr[r] .. ptr[r + 1]).
- * pgx_plan_missing_genome: missing[r] = the one genome gene genes[r] (present in N - 1 genomes) lacks. */
-int pgx_plan_coo_to_csr(const int32_t *row, const int32_t *col, int64_t nnz, int32_t n_genes, int32_t n_genomes,
-                        int64_t *indptr, int32_t *indices, int32_t *colsum, int64_t *n_duplicates,
-                        int32_t n_threads);
-int pgx_plan_folded_lists(const int64_t *indptr, const int32_t *indices, const int64_t *genes,
-                          const uint8_t *use_abs, const int64_t *ptr, int64_t n_rows, int32_t n_genomes,
-                          int32_t *flat, int32_t n_threads);
-int pgx_plan_missing_genome(const int64_t *indptr, const int32_t *indices, const int64_t *genes, int64_t n_rows,
-                            int32_t n_genomes, int32_t *missing, int32_t n_threads);
-/* Host-side helper of the planner: the order of the list rows inside their classes (rows of one chunk count and
- * list kind, consecutive in genes / use_abs / class_key) that balances, per group of ``modulus`` consecutive rows,
- * how many entries fall on each shared-memory bank residue (genome index modulo ``modulus``): such a group needs at
- * least max-over-residues(entries of the residue) gather steps however pgx_plan_bank_order arranges them.
- * order[i] (int64 [n_rows]) = current position of the row that takes place i.  Deterministic; ``window`` = candidates
- * looked at per choice (pangenomix_b200/plan.py, _balanced_row_order, is the numpy specification). */
-int pgx_plan_balance_rows(const int64_t *indptr, const int32_t *indices, const int64_t *genes,
-                          const uint8_t *use_abs, const int64_t *class_key, int64_t n_rows, int32_t n_genomes,
-                          int32_t modulus, int32_t window, int64_t *order, int32_t n_threads);
 /* Returns 1 when every 64-bit word of words[0 .. n) equals ``value``, else 0: the planner's "every stored value
  * is 1" test for the int64 (value 1) and float64 (value = bits of 1.0) ``data`` arrays of a table. */
 int pgx_plan_all_equal_u64(const uint64_t *words, int64_t n, uint64_t value, int32_t n_threads);

@@ -19,8 +19,7 @@ EXPORTS = (
     "pgx_launch_count", "pgx_bernoulli_scratch_bytes", "pgx_bernoulli_ll_grad",
     "pgx_legacy_shuffles", "pgx_profile_enable", "pgx_profile_read",
     "pgx_heaps_scratch_bytes", "pgx_heaps_fit", "pgx_estimate_pan_core",
-    "pgx_plan_bank_order", "pgx_plan_build_bitmap", "pgx_plan_coo_to_csr", "pgx_plan_folded_lists",
-    "pgx_plan_missing_genome", "pgx_plan_all_equal_u64", "pgx_plan_balance_rows", "pgx_inflate_raw",
+    "pgx_plan_all_equal_u64", "pgx_inflate_raw",
     "pgx_expand_deltas", "pgx_host_plan_create", "pgx_host_plan_destroy", "pgx_plan_create", "pgx_plan_upload",
     "pgx_plan_destroy", "pgx_set_trace", "pgx_legacy_random_raw", "pgx_coo_marginals", "pgx_frequency_spectrum",
     "pgx_coo_marginals_host", "pgx_ks_scratch_bytes", "pgx_ks_montecarlo", "pgx_ks_montecarlo_host", "pgx_expand_split", "pgx_split_head",
@@ -132,18 +131,6 @@ def load():
     lib.pgx_bernoulli_scratch_bytes.argtypes = [i64, i64]
     lib.pgx_bernoulli_ll_grad.restype = ctypes.c_int
     lib.pgx_bernoulli_ll_grad.argtypes = [vp, i64, i64, i64, vp, vp, vp, vp, vp, vp, vp, vp]
-    lib.pgx_plan_build_bitmap.restype = ctypes.c_int
-    lib.pgx_plan_build_bitmap.argtypes = [vp, vp, vp, i64, i32, i32, vp, i32]
-    lib.pgx_plan_bank_order.restype = ctypes.c_int
-    lib.pgx_plan_bank_order.argtypes = [vp, vp, i64, vp, vp, vp, vp, i64, i32, i32, i32, vp, i32]
-    lib.pgx_plan_coo_to_csr.restype = ctypes.c_int
-    lib.pgx_plan_coo_to_csr.argtypes = [vp, vp, i64, i32, i32, vp, vp, vp, ctypes.POINTER(i64), i32]
-    lib.pgx_plan_folded_lists.restype = ctypes.c_int
-    lib.pgx_plan_folded_lists.argtypes = [vp, vp, vp, vp, vp, i64, i32, vp, i32]
-    lib.pgx_plan_missing_genome.restype = ctypes.c_int
-    lib.pgx_plan_missing_genome.argtypes = [vp, vp, vp, i64, i32, vp, i32]
-    lib.pgx_plan_balance_rows.restype = ctypes.c_int
-    lib.pgx_plan_balance_rows.argtypes = [vp, vp, vp, vp, vp, i64, i32, i32, i32, vp, i32]
     lib.pgx_plan_all_equal_u64.restype = ctypes.c_int
     lib.pgx_plan_all_equal_u64.argtypes = [vp, i64, ctypes.c_uint64, i32]
     lib.pgx_inflate_raw.restype = ctypes.c_int

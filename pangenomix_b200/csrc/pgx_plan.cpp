@@ -1,12 +1,8 @@
-// Host-side helper of the planner (pangenomix_b200/plan.py): the bank ordering of the list rows.
-//
-// plan._bank_ordered_chunks decides, for every list row (the folded genome list of one gene, see
-// include/pgx.h), which entry sits at which gather step so that the lanes of a shared-memory
-// wavefront of list_kernel hit distinct banks of the rank table.  The numpy version in plan.py is
-// the specification (and stays, as the cross-check of the tests); this is the same algorithm --
-// same greedy edge colouring, same tie breaks, bit-identical output -- as plain loops over the
-// sub-blocks, spread over host threads.  It is O(slots) and removes three quarters of the planning
-// time of large tables.  Nothing here touches the GPU.
+// Threaded host steps of the planner (pgx_host_plan_create, pgx_plan_build.cpp): the table ingest (COO -> canonical
+// gene-major CSR), the folded lists, the missing genome of the single-absence rows, the residue-balanced order of the
+// list rows, the bank ordering of their entries and the bit-sliced bitmap of the long rows.  They are internal to the
+// library (namespace pgx); oracle/plan_np.py restates every step in numpy and the tests compare the two plans bit for
+// bit.  Only pgx_plan_all_equal_u64 is part of the C ABI.  Nothing here touches the GPU.
 #include <limits.h>
 #include <stdint.h>
 #include <stdlib.h>
@@ -26,7 +22,6 @@
 
 namespace pgx {
 int fail(int code, const char *fmt, ...);
-}
 
 namespace {
 
@@ -38,7 +33,7 @@ struct Group {
     std::vector<int8_t> res_at, pad_res;   // [lane][step]
 };
 
-// plan._colour_groups for one group: greedy edge colouring of lanes x residues with n_steps colours.
+// oracle/plan_np.py, _colour_groups, for one group: greedy edge colouring of lanes x residues with n_steps colours.
 // Same choices as the numpy specification (first maximum wins, stable order of the lanes), found with
 // less work: the residues a lane still holds are a bit mask, so a lane scans only those; the lane order
 // by slack is kept between steps (a lane's slack changes by at most one per step) and repaired by an
@@ -121,7 +116,7 @@ void colour(Group &g)
     }
 }
 
-// plan._positional_groups for one group.
+// oracle/plan_np.py, _positional_groups, for one group.
 void positional(Group &g)
 {
     const int R = g.r_mod, S = g.n_steps;
@@ -145,7 +140,17 @@ void positional(Group &g)
 
 }  // namespace
 
-extern "C" int pgx_plan_bank_order(const int32_t *flat, const int64_t *ptr, int64_t n_rows,
+// The bank ordering of the list rows (oracle/plan_np.py, _bank_ordered_chunks): which entry of a list row sits at which
+// gather step, so that the lanes of a shared-memory wavefront of list_kernel hit distinct banks of the rank table.  The
+// same greedy edge colouring, tie breaks and output as the numpy specification, as plain loops over the sub-blocks,
+// spread over host threads; the layout is the one struct pgx_plan documents.
+//   flat / ptr        : sorted folded lists of the n_rows list rows, concatenated (int32) / offsets (int64)
+//   block_*           : per sub-block of 32 rows: first chunk, chunks per row, first row, rows (int64 [n_blocks])
+//   modulus           : lanes per 128-byte wavefront: 8, 16 or 32 (= 64 / perms_per_cta, capped)
+//   colour_max_chunks : rows of more chunks use the cheap positional order instead of the edge colouring
+//   chunks            : out, uint16 [sum(block_nch) * 32 * 8]
+//   n_threads         : host threads (0 = choose)
+int pgx_plan_bank_order(const int32_t *flat, const int64_t *ptr, int64_t n_rows,
                                    const int64_t *block_first, const int64_t *block_nch,
                                    const int64_t *block_first_row, const int64_t *block_rows, int64_t n_blocks,
                                    int32_t n_genomes, int32_t modulus, int32_t colour_max_chunks,
@@ -227,7 +232,7 @@ extern "C" int pgx_plan_bank_order(const int32_t *flat, const int64_t *ptr, int6
 // The bit-sliced bitmap of the long rows (struct pgx_plan, d_bits): bit b of word
 // (sb * n_genomes + c) * 32 W + w is the presence of long row sb * 1024 W + 32 w + b in genome c.
 // ``bits`` must be zero-initialised; superblocks are independent and spread over host threads.
-extern "C" int pgx_plan_build_bitmap(const int64_t *indptr, const int32_t *indices, const int64_t *long_gene,
+int pgx_plan_build_bitmap(const int64_t *indptr, const int32_t *indices, const int64_t *long_gene,
                                      int64_t n_long, int32_t n_genomes, int32_t slice_words, uint32_t *bits,
                                      int32_t n_threads)
 {
@@ -274,7 +279,7 @@ extern "C" int pgx_plan_build_bitmap(const int64_t *indptr, const int32_t *indic
 // Table ingest: ``df_genes.data`` (scipy COO, gene x genome) -> canonical gene-major CSR, the
 // folded lists of the list rows and the missing genome of the single-absence rows.  These replace
 // scipy's single-threaded coo_tocsr / sum_duplicates / sort_indices and a few O(nnz) numpy
-// gathers of plan.py (which stay as the specification, PGX_PLAN_NUMPY=1) with threaded loops.
+// gathers of the specification (oracle/plan_np.py) with threaded loops.
 // ---------------------------------------------------------------------------------------------
 namespace {
 
@@ -329,7 +334,7 @@ void run_threads(int threads, F &&body)
 //           genome bitmap, short ones with std::sort -- and count duplicates; column sums.
 // Duplicate (gene, genome) pairs are kept and counted in *n_duplicates: scipy would sum them to 2, i.e.
 // a non-binary table.
-extern "C" int pgx_plan_coo_to_csr(const int32_t *row, const int32_t *col, int64_t nnz, int32_t n_genes,
+int pgx_plan_coo_to_csr(const int32_t *row, const int32_t *col, int64_t nnz, int32_t n_genes,
                                    int32_t n_genomes, int64_t *indptr, int32_t *indices, int32_t *colsum,
                                    int64_t *n_duplicates, int32_t n_threads)
 {
@@ -529,9 +534,9 @@ extern "C" int pgx_plan_coo_to_csr(const int32_t *row, const int32_t *col, int64
     return PGX_OK;
 }
 
-// plan._folded_lists: row r of the list rows is gene genes[r]; its folded list -- the present genomes
+// oracle/plan_np.py, _folded_lists: row r of the list rows is gene genes[r]; its folded list -- the present genomes
 // (use_abs[r] == 0) or the absent ones -- goes to flat[ptr[r] .. ptr[r + 1]), ascending.
-extern "C" int pgx_plan_folded_lists(const int64_t *indptr, const int32_t *indices, const int64_t *genes,
+int pgx_plan_folded_lists(const int64_t *indptr, const int32_t *indices, const int64_t *genes,
                                      const uint8_t *use_abs, const int64_t *ptr, int64_t n_rows,
                                      int32_t n_genomes, int32_t *flat, int32_t n_threads)
 {
@@ -579,7 +584,7 @@ extern "C" int pgx_plan_folded_lists(const int64_t *indptr, const int32_t *indic
 }
 
 // The one genome every gene of ``genes`` (present in exactly N - 1 genomes) is absent from.
-extern "C" int pgx_plan_missing_genome(const int64_t *indptr, const int32_t *indices, const int64_t *genes,
+int pgx_plan_missing_genome(const int64_t *indptr, const int32_t *indices, const int64_t *genes,
                                        int64_t n_rows, int32_t n_genomes, int32_t *missing, int32_t n_threads)
 {
     if (n_rows < 0 || n_genomes < 1) return pgx::fail(PGX_ERR_INVALID, "bad shape passed to pgx_plan_missing_genome");
@@ -612,23 +617,7 @@ extern "C" int pgx_plan_missing_genome(const int64_t *indptr, const int32_t *ind
     return PGX_OK;
 }
 
-// 1 when every 64-bit word of ``words`` equals ``value`` (the planner's "all stored values are 1" test for
-// int64 and float64 tables), else 0.
-extern "C" int pgx_plan_all_equal_u64(const uint64_t *words, int64_t n, uint64_t value, int32_t n_threads)
-{
-    if (n <= 0 || !words) return n <= 0 ? 1 : 0;
-    const int threads = host_threads(n_threads, std::max<long long>(1, n / (1 << 18)));
-    std::atomic<int> differs{0};
-    run_threads(threads, [&](int t) {
-        const int64_t lo = n * t / threads, hi = n * (t + 1) / threads;
-        uint64_t acc = 0;
-        for (int64_t i = lo; i < hi; ++i) acc |= words[i] ^ value;
-        if (acc) differs.store(1);
-    });
-    return differs.load() ? 0 : 1;
-}
-
-// plan._balanced_row_order: which list rows share a shared-memory wavefront group.  The lanes of a group
+// oracle/plan_np.py, _balanced_row_order: which list rows share a shared-memory wavefront group.  The lanes of a group
 // (``modulus`` consecutive rows of a sub-block) gather in lock step, one entry each, and two entries collide
 // when their genome indices agree modulo ``modulus``: a group needs at least max over residues of (entries of
 // that residue in the group) steps, however well pgx_plan_bank_order arranges them.  Rows may be put in any
@@ -639,7 +628,7 @@ extern "C" int pgx_plan_all_equal_u64(const uint64_t *words, int64_t n, uint64_t
 //   genes / use_abs / class_key : the list rows in their current order; rows of one class are consecutive
 //   order                       : out, int64 [n_rows]: position (in the current order) of the row that goes
 //                                 to each place of the new order
-extern "C" int pgx_plan_balance_rows(const int64_t *indptr, const int32_t *indices, const int64_t *genes,
+int pgx_plan_balance_rows(const int64_t *indptr, const int32_t *indices, const int64_t *genes,
                                      const uint8_t *use_abs, const int64_t *class_key, int64_t n_rows,
                                      int32_t n_genomes, int32_t modulus, int32_t window, int64_t *order,
                                      int32_t n_threads)
@@ -722,4 +711,22 @@ extern "C" int pgx_plan_balance_rows(const int64_t *indptr, const int32_t *indic
         }
     });
     return PGX_OK;
+}
+
+}  // namespace pgx
+
+// 1 when every 64-bit word of ``words`` equals ``value`` (the planner's "all stored values are 1" test for
+// int64 and float64 tables), else 0.
+extern "C" int pgx_plan_all_equal_u64(const uint64_t *words, int64_t n, uint64_t value, int32_t n_threads)
+{
+    if (n <= 0 || !words) return n <= 0 ? 1 : 0;
+    const int threads = pgx::host_threads(n_threads, std::max<long long>(1, n / (1 << 18)));
+    std::atomic<int> differs{0};
+    pgx::run_threads(threads, [&](int t) {
+        const int64_t lo = n * t / threads, hi = n * (t + 1) / threads;
+        uint64_t acc = 0;
+        for (int64_t i = lo; i < hi; ++i) acc |= words[i] ^ value;
+        if (acc) differs.store(1);
+    });
+    return differs.load() ? 0 : 1;
 }

@@ -5,7 +5,7 @@
 // matrix read_lsdf loads, sparse_utils.py:35) without Python: classification of the genes (closed forms, list
 // rows, bitmap rows), the order of the list rows, sub-blocks / runs / tasks, and -- through the threaded helpers
 // of pgx_plan.cpp -- the canonical CSR, the folded lists, the residue-balanced grouping, the bank ordering and the
-// bit-sliced bitmap.  pangenomix_b200/plan.py stays as the numpy SPECIFICATION of every step; the tests compare
+// bit-sliced bitmap.  oracle/plan_np.py is the numpy SPECIFICATION of every step; the tests compare
 // the two plans array by array, bit for bit.  Nothing here touches the GPU (pgx_plan_create in pgx_api.cu uploads
 // the image).
 #include <math.h>
@@ -24,7 +24,24 @@
 
 namespace pgx {
 int fail(int code, const char *fmt, ...);
-}
+
+// the threaded steps of pgx_plan.cpp (n_threads 0 = choose)
+int pgx_plan_coo_to_csr(const int32_t *row, const int32_t *col, int64_t nnz, int32_t n_genes, int32_t n_genomes,
+                        int64_t *indptr, int32_t *indices, int32_t *colsum, int64_t *n_duplicates, int32_t n_threads);
+int pgx_plan_missing_genome(const int64_t *indptr, const int32_t *indices, const int64_t *genes, int64_t n_rows,
+                            int32_t n_genomes, int32_t *missing, int32_t n_threads);
+int pgx_plan_build_bitmap(const int64_t *indptr, const int32_t *indices, const int64_t *long_gene, int64_t n_long,
+                          int32_t n_genomes, int32_t slice_words, uint32_t *bits, int32_t n_threads);
+int pgx_plan_balance_rows(const int64_t *indptr, const int32_t *indices, const int64_t *genes, const uint8_t *use_abs,
+                          const int64_t *class_key, int64_t n_rows, int32_t n_genomes, int32_t modulus, int32_t window,
+                          int64_t *order, int32_t n_threads);
+int pgx_plan_folded_lists(const int64_t *indptr, const int32_t *indices, const int64_t *genes, const uint8_t *use_abs,
+                          const int64_t *ptr, int64_t n_rows, int32_t n_genomes, int32_t *flat, int32_t n_threads);
+int pgx_plan_bank_order(const int32_t *flat, const int64_t *ptr, int64_t n_rows, const int64_t *block_first,
+                        const int64_t *block_nch, const int64_t *block_first_row, const int64_t *block_rows,
+                        int64_t n_blocks, int32_t n_genomes, int32_t modulus, int32_t colour_max_chunks,
+                        uint16_t *chunks, int32_t n_threads);
+}  // namespace pgx
 
 namespace {
 
@@ -122,7 +139,7 @@ extern "C" int pgx_host_plan_create(const int32_t *row, const int32_t *col, int6
         st->colsum.assign(static_cast<size_t>(n), 0);
         int64_t dups = 0;
         if (nnz > 0) {
-            if (int rc = pgx_plan_coo_to_csr(row, col, nnz, n_genes, n, indptr.data(), indices.data(), st->colsum.data(), &dups, 0))
+            if (int rc = pgx::pgx_plan_coo_to_csr(row, col, nnz, n_genes, n, indptr.data(), indices.data(), st->colsum.data(), &dups, 0))
                 return rc;
         }
         if (dups)
@@ -147,7 +164,7 @@ extern "C" int pgx_host_plan_create(const int32_t *row, const int32_t *col, int6
         }
         if (!single_a.empty()) {
             std::vector<int32_t> missing(single_a.size());
-            if (int rc = pgx_plan_missing_genome(indptr.data(), indices.data(), single_a.data(), static_cast<int64_t>(single_a.size()), n, missing.data(), 0))
+            if (int rc = pgx::pgx_plan_missing_genome(indptr.data(), indices.data(), single_a.data(), static_cast<int64_t>(single_a.size()), n, missing.data(), 0))
                 return rc;
             for (int32_t c : missing) ++st->w_absent[c];
         }
@@ -171,7 +188,7 @@ extern "C" int pgx_host_plan_create(const int32_t *row, const int32_t *col, int6
             });
             for (int64_t g : st->long_gene) nnz_long += m_of(g);
             st->bits.assign(static_cast<size_t>(n_super) * n * (sb_rows / 32), 0u);
-            if (int rc = pgx_plan_build_bitmap(indptr.data(), indices.data(), st->long_gene.data(), n_long, n, slice_words, st->bits.data(), 0))
+            if (int rc = pgx::pgx_plan_build_bitmap(indptr.data(), indices.data(), st->long_gene.data(), n_long, n, slice_words, st->bits.data(), 0))
                 return rc;
         }
 
@@ -209,7 +226,7 @@ extern "C" int pgx_host_plan_create(const int32_t *row, const int32_t *col, int6
         if (n_rows && !(no_balance && !strcmp(no_balance, "1"))) {
             std::vector<int64_t> class_key(static_cast<size_t>(n_rows)), order(static_cast<size_t>(n_rows));
             for (long long i = 0; i < n_rows; ++i) class_key[i] = n_chunk[i] * 2 + use_abs[i];
-            if (int rc = pgx_plan_balance_rows(indptr.data(), indices.data(), list_gene.data(), use_abs.data(), class_key.data(), n_rows, n,
+            if (int rc = pgx::pgx_plan_balance_rows(indptr.data(), indices.data(), list_gene.data(), use_abs.data(), class_key.data(), n_rows, n,
                                                modulus, std::max(BALANCE_WINDOW, 4 * modulus), order.data(), 0))
                 return rc;
             std::vector<int64_t> g2(static_cast<size_t>(n_rows)), l2(static_cast<size_t>(n_rows)), c2(static_cast<size_t>(n_rows));
@@ -232,7 +249,7 @@ extern "C" int pgx_host_plan_create(const int32_t *row, const int32_t *col, int6
         std::vector<int32_t> flat(static_cast<size_t>(ptr[n_rows]));
         long long nnz_list = 0;
         if (n_rows) {
-            if (int rc = pgx_plan_folded_lists(indptr.data(), indices.data(), list_gene.data(), use_abs.data(), ptr.data(), n_rows, n, flat.data(), 0))
+            if (int rc = pgx::pgx_plan_folded_lists(indptr.data(), indices.data(), list_gene.data(), use_abs.data(), ptr.data(), n_rows, n, flat.data(), 0))
                 return rc;
             for (int64_t g : list_gene) nnz_list += m_of(g);
         }
@@ -274,7 +291,7 @@ extern "C" int pgx_host_plan_create(const int32_t *row, const int32_t *col, int6
             if (at * CHUNK >= (1ll << 31)) return pgx::fail(PGX_ERR_UNSUPPORTED, "list rows too large for int32 chunk offsets");
             if (max_nch >= (1 << 16)) return pgx::fail(PGX_ERR_UNSUPPORTED, "list row too long for the task descriptor");
             st->chunks.resize(static_cast<size_t>(at) * CHUNK);
-            if (int rc = pgx_plan_bank_order(flat.data(), ptr.data(), n_rows, block_first.data(), b_nch.data(), b_first_row.data(), b_rows.data(),
+            if (int rc = pgx::pgx_plan_bank_order(flat.data(), ptr.data(), n_rows, block_first.data(), b_nch.data(), b_first_row.data(), b_rows.data(),
                                              n_blocks, n, modulus, COLOUR_MAX_CHUNKS, st->chunks.data(), 0))
                 return rc;
             phase("list rows: bank order");

@@ -63,7 +63,7 @@ void expand_split_rows(const uint8_t *rows, long long r0, long long r1, long lon
 
 namespace {
 
-constexpr int SENTINELS = 32;          // rank-table rows N .. N+31 hold 0xffff (plan.py)
+constexpr int SENTINELS = 32;          // rank-table rows N .. N+31 hold 0xffff (include/pgx.h)
 // Optional CUDA-event brackets around the kernels of every call (bench.py's roofline).
 struct ProfileEvents { cudaEvent_t begin, prep_done, list_done, probe_done, end; };
 bool g_profile_on = false;

@@ -12,7 +12,7 @@ import os
 import numpy as np
 
 from . import _native
-from .plan import HostPlan, build_host_plan
+from .plan import HostPlan, all_ones, build_host_plan
 
 
 def _torch():
@@ -151,24 +151,10 @@ class PanCoreEngine:
         self.c_plan = self._plan_ptr.contents
 
     def _upload(self, hp):
-        if hp.c_owner is not None:                       # the library's own planner made it: upload its image
-            host = hp.c_owner.pointer
-        else:                                            # numpy specification (tests, unusual tables): wrap the arrays
-            keep = [np.ascontiguousarray(a) for a in (
-                hp.chunks, hp.tasks, hp.sorted_idx, hp.sorted_ptr, hp.bits, hp.colsum, hp.w_present, hp.w_absent)]
-            ptr = [a.ctypes.data if a.size else None for a in keep]
-            image = _native.PgxHostPlan(
-                owner=None, chunks=ptr[0], tasks=ptr[1], sorted_idx=ptr[2], sorted_ptr=ptr[3], bits=ptr[4],
-                colsum=ptr[5], w_present=ptr[6], w_absent=ptr[7], row_gene=None, row_len=None, row_absent=None,
-                long_gene=None, nnz=hp.nnz, nnz_list=hp.nnz_list, nnz_long=hp.nnz_long, n_chunks=hp.n_chunks,
-                n_bits_words=int(hp.bits.size), n_sorted=int(hp.sorted_idx.size), n_genomes=hp.n_genomes,
-                n_genes=hp.n_genes, n_rows=hp.n_rows, n_tasks=hp.n_tasks, n_long=hp.n_long,
-                n_superblocks=hp.n_superblocks, perms_per_cta=hp.perms_per_cta, slice_words=hp.slice_words,
-                long_threshold=hp.long_threshold, max_colsum=int(hp.colsum.max()) if hp.colsum.size else 0,
-                n_empty=hp.n_empty, n_full=hp.n_full)
-            host = ctypes.pointer(image)
+        if hp.c_owner is None:
+            raise ValueError("host_plan must come from pangenomix_b200.plan.build_host_plan (the library's planner)")
         out = ctypes.POINTER(_native.PgxPlan)()
-        _native.check(self.lib.pgx_plan_upload(host, ctypes.byref(out)))
+        _native.check(self.lib.pgx_plan_upload(hp.c_owner.pointer, ctypes.byref(out)))
         return out
 
     def close(self):
@@ -426,13 +412,7 @@ def table_marginals(data, device=None, spectrum=True):
     n_genes, n_genomes = (int(v) for v in coo.shape)
     if n_genes > 2 ** 31 - 1 or n_genomes > 2 ** 31 - 1:
         raise ValueError("table too large")
-    values = np.asarray(coo.data)
-    if values.dtype in (np.dtype(np.int64), np.dtype(np.float64)) and values.flags.c_contiguous:
-        one = 1 if values.dtype == np.dtype(np.int64) else int(np.float64(1.0).view(np.uint64))
-        all_ones = bool(_native.load().pgx_plan_all_equal_u64(values.ctypes.data, values.shape[0], one, 0))
-    else:
-        all_ones = values.dtype != object and bool(np.all(values == 1))
-    if values.size and not all_ones:
+    if coo.nnz and not all_ones(coo.data):
         raise ValueError("table_marginals counts entries: every stored value must be 1 (binary presence/absence table)")
     row = np.ascontiguousarray(coo.row, dtype=np.int32)
     col = np.ascontiguousarray(coo.col, dtype=np.int32)

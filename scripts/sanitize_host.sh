@@ -26,7 +26,7 @@ for src in pgx_rng pgx_plan pgx_inflate pgx_expand pgx_plan_build; do
 done
 nvcc -O3 -std=c++17 -gencode arch=compute_100a,code=sm_100a -lineinfo -Xcompiler -fPIC,-O3,-pthread -shared \
   -I "$REPO/include" -I "$CSRC" -o "$OUT/libpgx_b200.so" \
-  "$CSRC/pgx_api.cu" "$CSRC/pgx_rarefy.cu" "$CSRC/pgx_bernoulli.cu" "$CSRC/pgx_heaps.cu" "$CSRC/pgx_betabin.cu" "$OUT/pgx_rng.o" "$OUT/pgx_plan.o" "$OUT/pgx_inflate.o" "$OUT/pgx_expand.o" "$OUT/pgx_plan_build.o" \
+  "$CSRC/pgx_api.cu" "$CSRC/pgx_rarefy.cu" "$CSRC/pgx_bernoulli.cu" "$CSRC/pgx_heaps.cu" "$CSRC/pgx_betabin.cu" "$CSRC/pgx_perm.cu" "$OUT/pgx_rng.o" "$OUT/pgx_plan.o" "$OUT/pgx_inflate.o" "$OUT/pgx_expand.o" "$OUT/pgx_plan_build.o" \
   $LINK
 cd "$REPO"
 if [ $# -eq 0 ]; then set -- tests/test_plan.py tests/test_abi_cpu.py tests/test_sparse_utils.py tests/test_distributed_cpu.py; fi

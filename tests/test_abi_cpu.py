@@ -20,7 +20,7 @@ def test_library_exports_every_declared_symbol():
     lib = _native.load()
     for name in declared:
         assert hasattr(lib, name), name
-    assert lib.pgx_version() == 320
+    assert lib.pgx_version() == 321
 
 
 def test_plan_struct_layout_matches_header():

@@ -1,10 +1,12 @@
-"""Host planning (pangenomix_b200/plan.py) checked on the CPU against the golden curves by
-walking the plan exactly as the kernels do (tests/plan_emulator.py)."""
+"""Host planning (pgx_host_plan_create through pangenomix_b200/plan.py) checked on the CPU against the golden
+curves by walking the plan exactly as the kernels do (tests/plan_emulator.py), and against the numpy
+specification of the planner (oracle/plan_np.py)."""
 import numpy as np
 import pytest
 import scipy.sparse
 
 from conftest import CURVE_CASES, draw_perms, golden_matrix, load_golden
+from oracle import plan_np
 from pangenomix_b200.plan import build_host_plan
 from plan_emulator import check_layout, curves_from_plan
 
@@ -91,23 +93,19 @@ def test_plan_bitmap_slices_of_1_2_4_words(slice_words):
 
 
 @pytest.mark.parametrize("perms_per_cta", [8, 4, 2])
-def test_plan_native_bank_order_equals_numpy_specification(monkeypatch, perms_per_cta):
-    """pgx_plan_bank_order (C++, threaded) must reproduce plan._bank_ordered_chunks_numpy bit for bit:
+def test_plan_native_bank_order_equals_specification(perms_per_cta):
+    """The library's bank ordering (C++, threaded) must reproduce plan_np._bank_ordered_chunks bit for bit:
     the colouring for short rows, the positional order for long ones, pads, ragged sub-blocks."""
     x = _mixed_matrix(1300, seed=31, per_class=90)
     coo = scipy.sparse.coo_matrix(x)
     native = build_host_plan(coo, long_threshold=0, perms_per_cta=perms_per_cta)
-    monkeypatch.setenv("PGX_PLAN_NUMPY", "1")
-    spec = build_host_plan(coo, long_threshold=0, perms_per_cta=perms_per_cta)
+    spec = plan_np.build_host_plan(coo, long_threshold=0, perms_per_cta=perms_per_cta)
     assert (native.tasks[:, 1] & 0xFFFF).max() > 32 > (native.tasks[:, 1] & 0xFFFF).min()      # both orderings in play
     assert np.array_equal(native.chunks, spec.chunks)
     assert np.array_equal(native.tasks, spec.tasks)
-    monkeypatch.delenv("PGX_PLAN_NUMPY")
     for w in (1, 2, 4):
         a = build_host_plan(coo, long_threshold=5, slice_words=w)
-        monkeypatch.setenv("PGX_PLAN_NUMPY", "1")
-        b = build_host_plan(coo, long_threshold=5, slice_words=w)
-        monkeypatch.delenv("PGX_PLAN_NUMPY")
+        b = plan_np.build_host_plan(coo, long_threshold=5, slice_words=w)
         assert a.n_long > 0 and np.array_equal(a.bits, b.bits) and np.array_equal(a.chunks, b.chunks)
 
 
@@ -160,8 +158,8 @@ def _plans_equal(a, b):
 
 @pytest.mark.parametrize("order", ["column-major", "row-major", "shuffled"])
 @pytest.mark.parametrize("shape", [(360, 700), (5000, 90), (70000, 12)])
-def test_plan_native_ingest_equals_scipy_specification(monkeypatch, order, shape):
-    """pgx_plan_coo_to_csr / pgx_plan_folded_lists / pgx_plan_missing_genome (threaded C++) against the scipy +
+def test_plan_native_ingest_equals_scipy_specification(order, shape):
+    """The library's table ingest, folded lists and missing genomes (threaded C++) against the scipy +
     numpy specification of the same steps: whatever the order of the COO entries, the whole plan is identical.
     70,000 genes make the counting sort use blocks of 256 genes; (5000, 90) holds single-absence rows."""
     g, n = shape
@@ -174,12 +172,10 @@ def test_plan_native_ingest_equals_scipy_specification(monkeypatch, order, shape
         row, col = row[p], col[p]
     coo = scipy.sparse.coo_matrix((np.ones(row.shape[0], dtype=np.int64), (row, col)), shape=shape)
     native = build_host_plan(coo, long_threshold=9)
-    monkeypatch.setenv("PGX_PLAN_NUMPY", "1")
-    spec = build_host_plan(coo, long_threshold=9)
-    monkeypatch.delenv("PGX_PLAN_NUMPY")
+    spec = plan_np.build_host_plan(coo, long_threshold=9)
     _plans_equal(native, spec)
     assert native.w_absent.sum() > 0 or n > 100
-    # float / bool ones take the same fast path, CSR input the scipy path: same plan
+    # float ones take the same path, CSR input is made canonical first: same plan
     _plans_equal(build_host_plan(coo.astype(np.float64), long_threshold=9), spec)
     _plans_equal(build_host_plan(coo.tocsr(), long_threshold=9), spec)
 
@@ -187,51 +183,64 @@ def test_plan_native_ingest_equals_scipy_specification(monkeypatch, order, shape
 def test_plan_native_ingest_errors_and_corner_cases():
     import ctypes
     from pangenomix_b200 import _native
-    from pangenomix_b200.plan import canonical_csr
     lib = _native.load()
 
     def call(row, col, g, n):
         row, col = np.asarray(row, dtype=np.int32), np.asarray(col, dtype=np.int32)
-        indptr, indices = np.empty(g + 1, dtype=np.int64), np.empty(max(1, row.size), dtype=np.int32)
-        colsum, dups = np.empty(n, dtype=np.int32), ctypes.c_int64(-1)
-        rc = lib.pgx_plan_coo_to_csr(row.ctypes.data, col.ctypes.data, row.size, g, n, indptr.ctypes.data,
-                                     indices.ctypes.data, colsum.ctypes.data, ctypes.byref(dups), 3)
-        return rc, indptr, indices[:row.size], colsum, dups.value
+        out = ctypes.POINTER(_native.PgxHostPlan)()
+        rc = lib.pgx_host_plan_create(row.ctypes.data, col.ctypes.data, row.size, g, n, -1, 0, 0, ctypes.byref(out))
+        if rc == 0:
+            lib.pgx_host_plan_destroy(out)
+        return rc
 
-    rc, indptr, indices, colsum, dups = call([2, 0, 2, 0], [1, 3, 0, 2], 4, 5)
-    assert rc == 0 and dups == 0
-    assert indptr.tolist() == [0, 2, 2, 4, 4] and indices.tolist() == [2, 3, 0, 1] and colsum.tolist() == [1, 1, 1, 1, 0]
-    assert call([0, 0, 1], [1, 1, 0], 2, 3)[4] == 1                       # a duplicate pair is reported, not merged
-    assert call([0, 2], [0, 0], 2, 3)[0] != 0 and b"gene index" in lib.pgx_last_error()
-    assert call([0, -1], [0, 0], 2, 3)[0] != 0
-    assert call([0, 1], [0, 3], 2, 3)[0] != 0 and b"genome index" in lib.pgx_last_error()
-    assert call([], [], 3, 2)[1].tolist() == [0, 0, 0, 0]
-    # the Python wrapper: duplicates fall back to scipy (summed to 2 -> rejected), zeros are absences
+    hp = build_host_plan(scipy.sparse.coo_matrix((np.ones(4, dtype=np.int64), ([2, 0, 2, 0], [1, 3, 0, 2])), shape=(4, 5)))
+    assert hp.c_owner is not None and hp.colsum.tolist() == [1, 1, 1, 1, 0] and hp.n_empty == 2
+    lists = {int(g): hp.sorted_idx[hp.sorted_ptr[r]:hp.sorted_ptr[r + 1]].tolist() for r, g in enumerate(hp.row_gene)}
+    assert lists == {0: [2, 3], 2: [0, 1]}
+    assert call([0, 0, 1], [1, 1, 0], 2, 3) == 1                  # a duplicate pair: PGX_ERR_INVALID
+    assert call([0, 2], [0, 0], 2, 3) != 0 and b"gene index" in lib.pgx_last_error()
+    assert call([0, -1], [0, 0], 2, 3) != 0
+    assert call([0, 1], [0, 3], 2, 3) != 0 and b"genome index" in lib.pgx_last_error()
+    assert call([], [], 3, 2) == 0
+    # the Python front end: duplicates are summed to 2 -> rejected, zeros are absences
     with pytest.raises(ValueError):
-        canonical_csr(scipy.sparse.coo_matrix((np.ones(3), ([0, 0, 1], [1, 1, 0])), shape=(2, 3)))
-    indptr, indices, colsum, shape = canonical_csr(
-        scipy.sparse.coo_matrix((np.array([1, 0, 1]), ([0, 0, 1], [0, 1, 2])), shape=(2, 3)))
-    assert indptr.tolist() == [0, 1, 2] and indices.tolist() == [0, 2] and colsum.tolist() == [1, 0, 1] and shape == (2, 3)
-    # folded lists / missing genome reject rows that do not match their descriptors
-    ip, ix = np.array([0, 2, 3], dtype=np.int64), np.array([0, 2, 1], dtype=np.int32)
-    genes, ua = np.array([0, 1], dtype=np.int64), np.array([1, 0], dtype=np.uint8)
-    ptr, flat = np.array([0, 1, 2], dtype=np.int64), np.empty(2, dtype=np.int32)
-    assert lib.pgx_plan_folded_lists(ip.ctypes.data, ix.ctypes.data, genes.ctypes.data, ua.ctypes.data,
-                                     ptr.ctypes.data, 2, 3, flat.ctypes.data, 1) == 0
-    assert flat.tolist() == [1, 1]
-    bad_ptr = np.array([0, 2, 3], dtype=np.int64)
-    assert lib.pgx_plan_folded_lists(ip.ctypes.data, ix.ctypes.data, genes.ctypes.data, ua.ctypes.data,
-                                     bad_ptr.ctypes.data, 2, 3, np.empty(3, dtype=np.int32).ctypes.data, 1) != 0
-    miss = np.empty(2, dtype=np.int32)
-    assert lib.pgx_plan_missing_genome(ip.ctypes.data, ix.ctypes.data, genes.ctypes.data, 1, 3, miss.ctypes.data, 1) == 0
-    assert miss[0] == 1
-    assert lib.pgx_plan_missing_genome(ip.ctypes.data, ix.ctypes.data, genes.ctypes.data, 2, 3, miss.ctypes.data, 1) != 0
+        build_host_plan(scipy.sparse.coo_matrix((np.ones(3), ([0, 0, 1], [1, 1, 0])), shape=(2, 3)))
+    hp = build_host_plan(scipy.sparse.coo_matrix((np.array([1, 0, 1]), ([0, 0, 1], [0, 1, 2])), shape=(2, 3)))
+    assert (hp.n_genes, hp.n_genomes, hp.nnz) == (2, 3, 2)
+    assert hp.colsum.tolist() == [1, 0, 1] and hp.w_present.tolist() == [1, 0, 1]
+
+
+def _input_formats(coo):
+    x = coo.toarray()
+    zeros = scipy.sparse.coo_matrix((np.concatenate([coo.data, np.zeros(5, dtype=coo.data.dtype)]),
+                                     (np.concatenate([coo.row, np.arange(5)]), np.concatenate([coo.col, np.full(5, 7)]))),
+                                    shape=coo.shape)
+    assert zeros.nnz == coo.nnz + 5 and not np.any(x[np.arange(5), 7])
+    return {"int64": coo.astype(np.int64), "float64": coo.astype(np.float64), "bool": coo.astype(bool),
+            "explicit-zeros": zeros, "csr": coo.tocsr(), "csc": coo.tocsc(), "dense": x,
+            "no-entries": scipy.sparse.coo_matrix(coo.shape, dtype=np.int64)}
+
+
+@pytest.mark.parametrize("fmt", ["int64", "float64", "bool", "explicit-zeros", "csr", "csc", "dense", "no-entries"])
+def test_every_input_format_is_planned_by_the_library(fmt):
+    """Whatever form the table comes in, the plan is the library's own (c_owner set) and equals the
+    specification array by array."""
+    coo = scipy.sparse.coo_matrix(_mixed_matrix(300, seed=17, per_class=30))
+    data = _input_formats(coo)[fmt]
+    hp = build_host_plan(data, long_threshold=12)
+    assert hp.c_owner is not None
+    spec = plan_np.build_host_plan(data, long_threshold=12)
+    _plans_equal(hp, spec)
+    if fmt == "no-entries":
+        assert hp.n_empty == coo.shape[0]
+    else:
+        assert hp.nnz == coo.nnz and hp.n_rows > 0 and hp.n_long > 0
 
 
 def test_plan_row_balance_lowers_bank_conflicts(monkeypatch):
-    """Rows are grouped so that the bank residues of a wavefront group are balanced (_balanced_row_order):
+    """Rows are grouped so that the bank residues of a wavefront group are balanced (plan_np._balanced_row_order):
     same rows, same curves, fewer shared-memory wavefronts per gather step than with rows sorted by length;
-    the C++ helper and the numpy specification agree on the order."""
+    the library and the numpy specification agree on the order."""
     import oracle
     from pangenomix_b200 import synth
     coo = synth.bernoulli_matrix(6000, 1500, 450, seed=3)          # thousands of short rows, hundreds per class
@@ -246,23 +255,19 @@ def test_plan_row_balance_lowers_bank_conflicts(monkeypatch):
     perms = draw_perms(5, 1500, 2)
     pan, core = oracle.pan_core_curves_minrank(coo, perms)
     assert np.array_equal(curves_from_plan(balanced, perms), np.hstack([pan, core]).astype(np.int64))
-    monkeypatch.setenv("PGX_PLAN_NUMPY", "1")
-    spec = build_host_plan(coo, long_threshold=100, perms_per_cta=8)
-    monkeypatch.delenv("PGX_PLAN_NUMPY")
+    spec = plan_np.build_host_plan(coo, long_threshold=100, perms_per_cta=8)
     _plans_equal(balanced, spec)
     # wide wavefront groups (16 and 32 lanes) and a window larger than a class
     for b in (4, 2):
         a = build_host_plan(coo, long_threshold=30, perms_per_cta=b)
-        monkeypatch.setenv("PGX_PLAN_NUMPY", "1")
-        c = build_host_plan(coo, long_threshold=30, perms_per_cta=b)
-        monkeypatch.delenv("PGX_PLAN_NUMPY")
+        c = plan_np.build_host_plan(coo, long_threshold=30, perms_per_cta=b)
         _plans_equal(a, c)
         check_layout(a)
 
 
 def test_plan_wide_table_two_permutations_per_cta_with_row_balance():
     """A C5-like width (50,000 genomes: 2 permutations per CTA, 32-lane wavefront groups, bitmap rows and list
-    rows side by side) through the planner's native helpers with the residue-balanced row order: the layout
+    rows side by side) through the library's planner with the residue-balanced row order: the layout
     invariants hold and the emulated kernels reproduce the oracle's curves."""
     from oracle import cport
     from pangenomix_b200 import synth
@@ -277,24 +282,17 @@ def test_plan_wide_table_two_permutations_per_cta_with_row_balance():
 
 
 @pytest.mark.parametrize("name", ["c1", "c2"])
-def test_three_planners_agree(monkeypatch, name):
-    """The library's own planner (pgx_host_plan_create, what a C host gets), the Python orchestration over the
-    library's per-step helpers (PGX_PLAN_PYTHON=1) and the numpy / scipy specification (PGX_PLAN_NUMPY=1): the same
-    plan, array by array, on configs C1 and C2."""
+def test_library_planner_equals_specification(name):
+    """The library's own planner (pgx_host_plan_create, what a C host gets) and the numpy / scipy specification
+    (oracle/plan_np.py): the same plan, array by array, on configs C1 and C2."""
     from conftest import config_matrix_cached
     from pangenomix_b200 import synth
     coo = synth.config_matrix("c1") if name == "c1" else config_matrix_cached("c2")
     library = build_host_plan(coo)
     assert library.c_owner is not None and library.n_long > 0 and library.n_rows > 0
-    monkeypatch.setenv("PGX_PLAN_PYTHON", "1")
-    helpers = build_host_plan(coo)
-    monkeypatch.delenv("PGX_PLAN_PYTHON")
-    monkeypatch.setenv("PGX_PLAN_NUMPY", "1")
-    spec = build_host_plan(coo)
-    monkeypatch.delenv("PGX_PLAN_NUMPY")
-    assert helpers.c_owner is None and spec.c_owner is None
+    spec = plan_np.build_host_plan(coo)
+    assert spec.c_owner is None
     _plans_equal(library, spec)
-    _plans_equal(helpers, spec)
     for f in ("n_empty", "n_full", "nnz", "nnz_list", "nnz_long", "long_threshold", "perms_per_cta", "slice_words"):
         assert getattr(library, f) == getattr(spec, f), f
     assert np.array_equal(library.row_gene, spec.row_gene) and np.array_equal(library.long_gene, spec.long_gene)
