@@ -155,7 +155,11 @@ int pgx_pan_core_curves(const pgx_plan *plan, const uint16_t *d_perms, int64_t n
                         int32_t *d_curves, void *stream);
 
 /* Same, float64 output exactly as the reference's DataFrame values (:76-77, :97).
- * d_hist is caller scratch of n_perm * 2N int32. */
+ *   d_hist   : caller scratch of n_perm * 2N int32, 4-byte aligned (the kernels read and write it as uint16 and
+ *              32-bit words and use 16-byte accesses only where they find it 16-byte aligned); overwritten
+ *   d_curves : [n_perm][2N] float64, 8-byte aligned (16-byte stores where the rows are 16-byte aligned, else 8-byte);
+ *              must not overlap d_hist
+ * n_perm == 0 writes nothing and returns PGX_OK.  Asynchronous on ``stream``. */
 int pgx_pan_core_curves_f64(const pgx_plan *plan, const uint16_t *d_perms, int64_t n_perm,
                             int32_t *d_hist, double *d_curves, void *stream);
 
@@ -192,9 +196,11 @@ int pgx_set_tuning(int32_t perms_per_cta, int32_t row_splits, int32_t threads_pe
 
 /* Per-kernel timing for roofline reports: while enabled, every pgx_pan_core_curves[_f64]
  * call brackets its kernels with CUDA events on the caller's stream and runs the two row kernels
- * back to back.  pgx_profile_read waits for them, returns the summed durations (ms) of the list
- * kernel, the bitmap-probe kernel and everything else (prep + scan kernels) and the number of
- * calls since the last read, and releases the events. */
+ * back to back.  The host-buffer calls (pgx_pan_core_curves_host, pgx_estimate_pan_core) are never
+ * profiled, whatever the table's bin format, and keep their schedule.  pgx_profile_read waits for the
+ * events, returns the summed durations (ms) of the list kernel, the bitmap-probe kernel (a kernel a
+ * call did not launch, because the table has no such rows, counts 0) and everything else (prep + scan
+ * kernels) and the number of profiled calls since the last read, and releases the events. */
 int pgx_profile_enable(int32_t on);
 int pgx_profile_read(double *list_ms, double *probe_ms, double *scan_ms, int64_t *calls);
 

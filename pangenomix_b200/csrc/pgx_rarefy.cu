@@ -64,8 +64,12 @@ void expand_split_rows(const uint8_t *rows, long long r0, long long r1, long lon
 namespace {
 
 constexpr int SENTINELS = 32;          // rank-table rows N .. N+31 hold 0xffff (include/pgx.h)
-// Optional CUDA-event brackets around the kernels of every call (bench.py's roofline).
-struct ProfileEvents { cudaEvent_t begin, prep_done, list_done, probe_done, end; };
+// Optional CUDA-event brackets around the kernels of every device-pointer call (bench.py's roofline).  A row kernel the
+// call did not launch counts 0 ms, not the gap between two events recorded back to back.
+struct ProfileEvents {
+    cudaEvent_t begin, prep_done, list_done, probe_done, end;
+    bool list_ran, probe_ran;
+};
 bool g_profile_on = false;
 std::mutex g_profile_mu;
 std::vector<ProfileEvents> g_profile_events;
@@ -1158,7 +1162,11 @@ int run_rows(const pgx_plan *plan, const uint16_t *d_perms, long long n_perm, co
         if (gate) work.started = aux->d_started;
         if (int rc = launch_list_b<P16>(*plan, d_perms, n_perm, work, lim, stream, &list_grid)) return rc;
     }
-    if (ev) PGX_CUDA(cudaEventRecord(ev->list_done, stream));
+    if (ev) {
+        ev->list_ran = plan->n_tasks > 0;
+        ev->probe_ran = plan->n_long > 0;
+        PGX_CUDA(cudaEventRecord(ev->list_done, stream));
+    }
     if (overlap) {
         // launched AFTER the list kernel: one list CTA per SM first, probe CTAs fill what is left
         if (gate) {
@@ -1199,9 +1207,10 @@ int launch_scan(const pgx_plan *plan, long long n_perm, const Work &work, OutT *
 }
 
 // Curves of n_perm permutations: d_work is an int32 [n_perm][2N] buffer (the output itself for OutT = int32).
+// ``profiled``: bracket the kernels with the events of pgx_profile_enable (the device-pointer calls only).
 template <typename OutT>
 int run_curves(const pgx_plan *plan, const uint16_t *d_perms, long long n_perm, int32_t *d_work,
-               OutT *d_out, cudaStream_t stream, Aux *own_aux = nullptr, int *d_bad_rows = nullptr)
+               OutT *d_out, cudaStream_t stream, bool profiled, Aux *own_aux = nullptr, int *d_bad_rows = nullptr)
 {
     if (int rc = check_plan(plan)) return rc;
     if (n_perm < 0) return fail(PGX_ERR_INVALID, "n_perm < 0");
@@ -1210,7 +1219,7 @@ int run_curves(const pgx_plan *plan, const uint16_t *d_perms, long long n_perm, 
     const long long n = plan->n_genomes;
     const bool p16 = packed_bins(plan);
     ProfileEvents ev{};
-    const bool profile = g_profile_on;
+    const bool profile = profiled && g_profile_on;
     if (profile) {
         PGX_CUDA(cudaEventCreate(&ev.begin));
         PGX_CUDA(cudaEventCreate(&ev.prep_done));
@@ -1555,9 +1564,11 @@ int host_pipeline(const pgx_plan *plan, const uint16_t *h_perms, uint32_t *mt_ke
                 rc = fail(PGX_ERR_CUDA, "D2H copy of the curve steps failed: %s", cudaGetErrorString(cudaGetLastError()));
         } else if (!rc) {
             s.head = 0;
-            rc = out_f64 ? run_curves<double>(plan, s.d_perm, cnt, reinterpret_cast<int32_t *>(s.d_hist), s.d_f64, s.stream, &s.aux, d_bad_rows)
+            // (host-buffer calls are never profiled, in either bin format: include/pgx.h)
+            rc = out_f64 ? run_curves<double>(plan, s.d_perm, cnt, reinterpret_cast<int32_t *>(s.d_hist), s.d_f64, s.stream, false,
+                                              &s.aux, d_bad_rows)
                          : run_curves<int32_t>(plan, s.d_perm, cnt, reinterpret_cast<int32_t *>(s.d_hist),
-                                               reinterpret_cast<int32_t *>(s.d_hist), s.stream, &s.aux, d_bad_rows);
+                                               reinterpret_cast<int32_t *>(s.d_hist), s.stream, false, &s.aux, d_bad_rows);
             const void *from = out_f64 ? static_cast<const void *>(s.d_f64) : static_cast<const void *>(s.d_hist);
             if (!rc && cudaMemcpyAsync(s.h_rows, from, out_elem * cnt * 2 * n, cudaMemcpyDeviceToHost, s.stream) != cudaSuccess)
                 rc = fail(PGX_ERR_CUDA, "D2H copy of the curves failed: %s", cudaGetErrorString(cudaGetLastError()));
@@ -1594,14 +1605,14 @@ int pgx_pan_core_curves(const pgx_plan *plan, const uint16_t *d_perms, int64_t n
                         int32_t *d_curves, void *stream)
 {
     return pgx::run_curves<int32_t>(plan, d_perms, n_perm, d_curves, d_curves,
-                                    static_cast<cudaStream_t>(stream));
+                                    static_cast<cudaStream_t>(stream), true);
 }
 
 int pgx_pan_core_curves_f64(const pgx_plan *plan, const uint16_t *d_perms, int64_t n_perm,
                             int32_t *d_hist, double *d_curves, void *stream)
 {
     return pgx::run_curves<double>(plan, d_perms, n_perm, d_hist, d_curves,
-                                   static_cast<cudaStream_t>(stream));
+                                   static_cast<cudaStream_t>(stream), true);
 }
 
 int pgx_pan_core_curves_host(const pgx_plan *plan, const uint16_t *h_perms, int64_t n_perm,
@@ -1646,8 +1657,8 @@ int pgx_profile_read(double *list_ms, double *probe_ms, double *scan_ms, int64_t
         PGX_CUDA(cudaEventElapsedTime(&t1, ev.prep_done, ev.list_done));
         PGX_CUDA(cudaEventElapsedTime(&t2, ev.list_done, ev.probe_done));
         PGX_CUDA(cudaEventElapsedTime(&t3, ev.probe_done, ev.end));
-        a += t1;
-        b += t2;
+        if (ev.list_ran) a += t1;
+        if (ev.probe_ran) b += t2;
         c += t0 + t3;                    // prep + scan: everything that is not a row kernel
         cudaEventDestroy(ev.begin);
         cudaEventDestroy(ev.prep_done);

@@ -333,14 +333,19 @@ def test_c4_full_size_properties_and_spot_parity(engine_mod):
     sample = np.r_[0:24, 488:512, 984:1000]                                 # 64 curves against the oracle's C port
     ref_pan, ref_core = cport.curves_direct(coo, perms[sample].astype(np.int32), n_threads=os.cpu_count() or 1)
     assert np.array_equal(curves[sample], np.hstack([ref_pan, ref_core]).astype(np.int32))
-    # per-kernel timing mode runs the row kernels back to back instead of side by side
+    # per-kernel timing mode runs the row kernels back to back instead of side by side (device calls only: host-buffer
+    # calls are never profiled)
+    import torch
+    _native.profile_read()
     _native.profile_enable(True)
     try:
-        again = eng.curves_host(perms[:200])
+        again = eng.curves_device(torch.from_numpy(perms[:200].view(np.int16)).cuda()).cpu().numpy()
+        assert _native.profile_read()[3] == 1
     finally:
         _native.profile_enable(False)
         _native.profile_read()
     assert np.array_equal(again, curves[:200])
+    assert np.array_equal(eng.curves_host(perms[:200]), curves[:200])
 
 
 def test_c5_full_size_spot_parity(engine_mod):
