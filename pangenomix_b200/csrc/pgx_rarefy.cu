@@ -23,7 +23,8 @@
 //   minima (VIMNMX.U16x2).  The host ordered the indices of a row so that the lanes of a
 //   wavefront hit distinct banks.  If the min is 0 the wanted statistic is the mex of the list's
 //   ranks instead: such (row, permutation) events are queued per warp and resolved 32 at a time
-//   against the sorted copy of the lists.
+//   against the sorted copy of the lists.  With packed bins the other minima of present lists are
+//   counted in shared memory once the item's gathers are done (see list_kernel).
 // Kernel 2 (probe_kernel<W>): genes with long lists, stored as a genome-major, bit-sliced
 //   bitmap (32 genes per word).  A warp walks one genome order for 1,024 W genes at once, one
 //   coalesced line of 128 W bytes per step; the first genome whose bit differs from the rank-0
@@ -400,6 +401,34 @@ __device__ __forceinline__ void gather_chunk(const uint16_t *table, const uint4 
     gather_min<B>(table, v.w >> 16, acc);
 }
 
+// The B minima of one list row, as the packed registers hold them, to and from the list kernel's scratch
+// (minima[slot][row][q]).  Evict-first both ways: the scratch streams through L2 while the probe kernel's bitmap is
+// meant to stay there.
+template <int B>
+__device__ __forceinline__ void store_minima(uint16_t *p, const uint32_t (&acc)[Packed<B>::REGS])
+{
+    if constexpr (B == 8) __stcs(reinterpret_cast<uint4 *>(p), make_uint4(acc[0], acc[1], acc[2], acc[3]));
+    else if constexpr (B == 4) __stcs(reinterpret_cast<uint2 *>(p), make_uint2(acc[0], acc[1]));
+    else if constexpr (B == 2) __stcs(reinterpret_cast<unsigned int *>(p), acc[0]);
+    else __stcs(reinterpret_cast<unsigned short *>(p), static_cast<unsigned short>(acc[0]));
+}
+
+template <int B>
+__device__ __forceinline__ void load_minima(const uint16_t *p, uint32_t (&m)[Packed<B>::REGS])
+{
+    if constexpr (B == 8) {
+        const uint4 v = __ldcs(reinterpret_cast<const uint4 *>(p));
+        m[0] = v.x; m[1] = v.y; m[2] = v.z; m[3] = v.w;
+    } else if constexpr (B == 4) {
+        const uint2 v = __ldcs(reinterpret_cast<const uint2 *>(p));
+        m[0] = v.x; m[1] = v.y;
+    } else if constexpr (B == 2) {
+        m[0] = __ldcs(reinterpret_cast<const unsigned int *>(p));
+    } else {
+        m[0] = __ldcs(reinterpret_cast<const unsigned short *>(p));
+    }
+}
+
 // mex of the ranks of a sorted genome list, given that rank 0 is in it: walk the genome
 // order from rank 1 and stop at the first genome that is not in the list.
 __device__ __noinline__ int mex_probe(const uint16_t *__restrict__ perm,
@@ -424,13 +453,23 @@ constexpr int EVENT_QUEUE = 64;
 // The chunk stream of a task is prefetched through THREE separately named buffers, each refilled by its own
 // load instruction: a rotating buffer refilled by ONE static LDG gets one scoreboard from the compiler, and waiting
 // for its oldest chunk then waits for every chunk load in flight (decoded from the SASS control bits of round 1's
-// kernel).  The end of a sub-block issues its B histogram updates back to back; the rare "min == 0" events are
-// collected in a per-lane mask and queued under one vote.  REGCAP x threads is sized so that CTAs of the probe
-// kernel, which runs beside this one on a second stream, find registers on every SM (48 x 1,024 or 64 x 768).
+// kernel).  The rare "min == 0" events are collected in a per-lane mask and queued under one vote.  REGCAP x threads
+// is sized so that CTAs of the probe kernel, which runs beside this one on a second stream, find registers on every
+// SM (48 x 1,024 or 64 x 768).
+//
+// Where the minima go.  Without ``minima`` (int32 bins, or a scratch too large) the end of a sub-block adds its B
+// minima straight into the global histogram rows: B REDs whose 32 lanes hit 32 unrelated lines, about 11 LSU
+// wavefronts each (29 % of the kernel's wavefronts on C4).  With ``minima`` (packed bins) a present-list sub-block
+// stores its minima to the CTA's slot of the scratch, minima[blockIdx.x][row][q] -- one coalesced store of 32 x 2B
+// bytes -- and once the item's gathers are done and the rank table is dead, its shared memory holds B packed pan-side
+// histograms: the item's minima are read back and counted with shared atomics, and the non-zero words are added
+// into the global rows with coalesced atomics (the probe kernel adds into the same rows).  A partial bin cannot
+// exceed the full one, so neither the shared nor the global words carry (the argument for packed bins).
+// Absent-list rows (about 1 % of C4's) and the mex events keep their global REDs.
 template <int B, int REGCAP, bool P16>
 __global__ void __maxnreg__(REGCAP)
 list_kernel(const pgx_plan plan, const uint16_t *__restrict__ perms, const long long n_perm,
-            const Work work, const int splits, const long long n_items)
+            const Work work, const int splits, const long long n_items, uint16_t *__restrict__ minima)
 {
     extern __shared__ __align__(16) uint16_t table[];   // [(N + 32)][B], then the warps' event queues
     __shared__ int s_next_task;
@@ -513,6 +552,8 @@ list_kernel(const pgx_plan plan, const uint16_t *__restrict__ perms, const long 
         PGX_DEVICE_CHECK(td.z >= 0 && td.z + n_rows <= plan.n_rows);
         uint32_t *list_hist = work.hist + p0 * work.hist_stride;
         const int side = absent_list ? n : 0;
+        // warp-uniform: this task's minima go to the scratch and are counted after the gathers
+        uint16_t *const slot = P16 && minima && !absent_list ? minima + static_cast<size_t>(blockIdx.x) * plan.n_rows * B : nullptr;
 
         uint32_t acc[REGS];
 #pragma unroll
@@ -528,6 +569,7 @@ list_kernel(const pgx_plan plan, const uint16_t *__restrict__ perms, const long 
             gather_chunk<B>(table, cur, acc);
             if (--left) return;
             const bool valid = rows_left > 0;
+            if (slot && valid) store_minima<B>(slot + static_cast<size_t>(row) * B, acc);
             uint32_t zero = 0;                            // bit q: this row's min under permutation q is 0
 #pragma unroll
             for (int q = 0; q < B; ++q) {
@@ -538,7 +580,7 @@ list_kernel(const pgx_plan plan, const uint16_t *__restrict__ perms, const long 
                     if (valid) {
                         // (mn >= n: a rank row with a hole, i.e. not a permutation -- counted nowhere, reported by the host calls)
                         if (mn == 0) zero |= 1u << q;
-                        else if (mn < static_cast<uint32_t>(n)) hist_add<P16>(list_hist + q * work.hist_stride, side + static_cast<int>(mn), 1u);
+                        else if (!slot && mn < static_cast<uint32_t>(n)) hist_add<P16>(list_hist + q * work.hist_stride, side + static_cast<int>(mn), 1u);
                     }
                 }
             }
@@ -591,6 +633,57 @@ list_kernel(const pgx_plan plan, const uint16_t *__restrict__ perms, const long 
     }
     if (lane < queued) resolve(queue[lane]);
     __syncthreads();                                      // every warp is done with this table
+
+    if constexpr (P16) {
+        if (minima) {
+            // ---- count the item's scratch minima in B packed pan-side histograms where the table was ----
+            uint32_t *s_hist = reinterpret_cast<uint32_t *>(table);            // [B][words]; pan bin k: half (k & 1) of word k >> 1
+            const int words = (n + 1) >> 1;
+            for (int i = tid; i < (B * words + 3) >> 2; i += blockDim.x)
+                reinterpret_cast<uint4 *>(s_hist)[i] = make_uint4(0u, 0u, 0u, 0u);
+            __syncthreads();
+            const uint16_t *__restrict__ slot = minima + static_cast<size_t>(blockIdx.x) * plan.n_rows * B;
+            constexpr int AHEAD = 4;                      // rows per lane in flight: the scratch comes back from HBM
+            for (long long t = tid >> 5;; t += blockDim.x >> 5) {
+                const long long task = t * splits + split;
+                if (task >= plan.n_tasks) break;
+                const int4 d = __ldg(tasks + task);
+                if (!(d.y & 0xffff) || ((d.y >> 24) & 1)) continue;            // absent lists were counted by REDs
+                const uint16_t *m = slot + static_cast<size_t>(d.z) * B;
+                for (int r0 = lane; r0 < d.w; r0 += 32 * AHEAD) {
+                    uint32_t v[AHEAD][REGS];
+#pragma unroll
+                    for (int j = 0; j < AHEAD; ++j) {
+                        if (r0 + 32 * j < d.w) {
+                            load_minima<B>(m + static_cast<size_t>(r0 + 32 * j) * B, v[j]);
+                        } else {
+#pragma unroll
+                            for (int i = 0; i < REGS; ++i) v[j][i] = 0xffffffffu;
+                        }
+                    }
+#pragma unroll
+                    for (int j = 0; j < AHEAD; ++j) {
+#pragma unroll
+                        for (int q = 0; q < B; ++q) {
+                            const uint32_t mn = B == 1 ? v[j][0] & 0xffffu : (v[j][q >> 1] >> ((q & 1) * 16)) & 0xffffu;
+                            // pan bins 1 .. N-1 only: 0 went to the mex queue, >= N is a rank row with a hole
+                            if (q < n_valid && mn - 1u < static_cast<uint32_t>(n - 1))
+                                atomicAdd(s_hist + q * words + (mn >> 1), 1u << ((mn & 1) * 16));
+                        }
+                    }
+                }
+            }
+            __syncthreads();
+            for (int q = 0; q < n_valid; ++q) {
+                uint32_t *dst = work.hist + (p0 + q) * work.hist_stride;
+                for (int w = tid; w < words; w += blockDim.x) {
+                    const uint32_t c = s_hist[q * words + w];
+                    if (c) atomicAdd(dst + w, c);
+                }
+            }
+            __syncthreads();                              // the next item's table overwrites the histograms
+        }
+    }
     }
     if (work.trace && tid == 0) trace_cta(work, 1u, t_start);
 }
@@ -959,6 +1052,35 @@ int list_variant()
     return v;
 }
 
+// Largest scratch of row minima one list launch takes (grid x n_rows x B x 2 bytes; C4: 244 MB, C5: 774 MB).
+constexpr size_t MINIMA_SCRATCH_MAX = size_t(1) << 30;
+
+// The scratch comes from a pool of the library's own per device that keeps its memory between launches: the device's
+// default pool hands freed memory back to the driver at every synchronisation, and the host-buffer calls synchronise
+// once per block.
+int scratch_pool(cudaMemPool_t *out)
+{
+    static std::mutex mu;
+    static cudaMemPool_t pools[64] = {};
+    int dev = 0;
+    PGX_CUDA(cudaGetDevice(&dev));
+    if (dev < 0 || dev >= 64) return fail(PGX_ERR_UNSUPPORTED, "device ordinal %d out of range", dev);
+    std::lock_guard<std::mutex> lock(mu);
+    if (!pools[dev]) {
+        cudaMemPoolProps props = {};
+        props.allocType = cudaMemAllocationTypePinned;
+        props.location.type = cudaMemLocationTypeDevice;
+        props.location.id = dev;
+        cudaMemPool_t pool = nullptr;
+        PGX_CUDA(cudaMemPoolCreate(&pool, &props));
+        uint64_t keep = ~uint64_t(0);
+        PGX_CUDA(cudaMemPoolSetAttribute(pool, cudaMemPoolAttrReleaseThreshold, &keep));
+        pools[dev] = pool;
+    }
+    *out = pools[dev];
+    return PGX_OK;
+}
+
 template <int B, bool P16>
 int launch_list(const pgx_plan &plan, const uint16_t *d_perms, long long n_perm, const Work &work,
                 const DeviceLimits &lim, cudaStream_t stream, unsigned *grid_out)
@@ -991,7 +1113,21 @@ int launch_list(const pgx_plan &plan, const uint16_t *d_perms, long long n_perm,
     PGX_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, smem));
     if (per_sm < 1) return fail(PGX_ERR_UNSUPPORTED, "list kernel does not fit an SM with %d threads", threads);
     const long long grid = max(1ll, min(n_items, static_cast<long long>(lim.sm_count) * max(1, per_sm)));
-    kernel<<<static_cast<unsigned>(grid), threads, smem, stream>>>(plan, d_perms, n_perm, work, splits, n_items);
+    // Packed bins: the row minima are counted in shared memory (list_kernel) through a scratch of one slot per CTA,
+    // taken stream-ordered for this launch.  Above MINIMA_SCRATCH_MAX, or when the pool has no room, the minima go
+    // to the global histogram rows directly.
+    uint16_t *minima = nullptr;
+    if (P16 && plan.n_rows > 0) {
+        const size_t bytes = static_cast<size_t>(grid) * static_cast<size_t>(plan.n_rows) * B * sizeof(uint16_t);
+        cudaMemPool_t pool = nullptr;
+        if (bytes <= MINIMA_SCRATCH_MAX &&
+            (scratch_pool(&pool) != PGX_OK || cudaMallocFromPoolAsync(reinterpret_cast<void **>(&minima), bytes, pool, stream) != cudaSuccess)) {
+            cudaGetLastError();
+            minima = nullptr;
+        }
+    }
+    kernel<<<static_cast<unsigned>(grid), threads, smem, stream>>>(plan, d_perms, n_perm, work, splits, n_items, minima);
+    if (minima) cudaFreeAsync(minima, stream);    // (an error of the launch stays the last error)
     PGX_LAUNCH_CHECK("list_kernel");
     if (grid_out) *grid_out = static_cast<unsigned>(grid);
     return PGX_OK;
