@@ -536,6 +536,35 @@ list_kernel(const pgx_plan plan, const uint16_t *__restrict__ perms, const long 
         // present list: min -> pan histogram, mex -> core histogram; absent list: swapped.
         if (k < n) hist_add<P16>(work.hist + (p0 + q) * work.hist_stride, ((ev & 8) ? 0 : n) + k, 1u);
     };
+    // Queue the events of one sub-block close (bit i: permutation 2i, bit 16 + i: permutation 2i + 1): lane l's events take the queue positions queued + (events of lanes < l)
+    // onwards, found with one exclusive scan over the warp (ballots of the bits of the per-lane count, at most 8).
+    // A close can bring 256 events: the queue is filled in rounds, and whenever it holds 32 or more, 32 are resolved,
+    // so that queued < 32 between closes and no position reaches EVENT_QUEUE.
+    auto queue_events = [&](uint32_t zero, const uint32_t tag) {
+        const uint32_t cnt = __popc(zero), below = (1u << lane) - 1u;
+        int at = queued, end = queued;
+#pragma unroll
+        for (int b = 0; b < 4; ++b) {
+            const uint32_t m = __ballot_sync(FULL_MASK, (cnt >> b) & 1u);
+            at += __popc(m & below) << b;
+            end += __popc(m) << b;
+        }
+        for (;;) {
+            while (zero && at < EVENT_QUEUE) {
+                const int bit = __ffs(zero) - 1;
+                zero &= zero - 1u;
+                queue[at++] = tag | static_cast<uint32_t>(((bit & 15) << 1) | (bit >> 4));
+            }
+            __syncwarp();
+            if (end < 32) break;
+            const uint32_t e = queue[min(end, EVENT_QUEUE) - 32 + lane];
+            __syncwarp();
+            resolve(e);
+            at -= 32;                                     // the queue keeps its min(end, EVENT_QUEUE) - 32 oldest entries
+            end -= 32;
+        }
+        queued = end;
+    };
 
     // A task is a run of consecutive sub-blocks (32 rows x nch chunks each) laid out back to
     // back, so the warp streams chunk iterations 0 .. n_sub * nch - 1 and closes a sub-block every
@@ -569,40 +598,33 @@ list_kernel(const pgx_plan plan, const uint16_t *__restrict__ perms, const long 
             gather_chunk<B>(table, cur, acc);
             if (--left) return;
             const bool valid = rows_left > 0;
-            if (slot && valid) store_minima<B>(slot + static_cast<size_t>(row) * B, acc);
-            uint32_t zero = 0;                            // bit q: this row's min under permutation q is 0
+            if (slot) {
+                // Packed close.  Permutations past n_valid and pad lanes gathered only 0xffff entries, so their minima
+                // are never 0.  zero: bit i for permutation 2i, bit 16 + i for permutation 2i + 1 (min 0).
+                if (valid) store_minima<B>(slot + static_cast<size_t>(row) * B, acc);
+                uint32_t zero = 0;
 #pragma unroll
-            for (int q = 0; q < B; ++q) {
-                if (q < n_valid) {
-                    uint32_t mn;
-                    if constexpr (B == 1) mn = acc[0] & 0xffffu;
-                    else mn = (acc[q >> 1] >> ((q & 1) * 16)) & 0xffffu;
-                    if (valid) {
-                        // (mn >= n: a rank row with a hole, i.e. not a permutation -- counted nowhere, reported by the host calls)
-                        if (mn == 0) zero |= 1u << q;
-                        else if (!slot && mn < static_cast<uint32_t>(n)) hist_add<P16>(list_hist + q * work.hist_stride, side + static_cast<int>(mn), 1u);
-                    }
-                }
-            }
-            // min == 0: the wanted statistic is the mex; queue (row, permutation), resolve 32 at a time
-            if (__any_sync(FULL_MASK, zero != 0)) {
-#pragma unroll 1
+                for (int i = 0; i < REGS; ++i) zero |= __vseteq2(acc[i], 0u) << i;
+                if constexpr (B == 1) zero &= 1u;                // the high half of a B = 1 minimum is 0
+                if (!valid) zero = 0;
+                if (__any_sync(FULL_MASK, zero != 0)) queue_events(zero, static_cast<uint32_t>(row) << 4);
+            } else {
+                uint32_t zero = 0;                        // the packed close's bit for permutation q: min 0
+#pragma unroll
                 for (int q = 0; q < B; ++q) {
-                    const bool ev = (zero >> q) & 1u;
-                    const uint32_t m = __ballot_sync(FULL_MASK, ev);
-                    if (!m) continue;
-                    PGX_DEVICE_CHECK(queued + __popc(m) <= EVENT_QUEUE);
-                    if (ev) queue[queued + __popc(m & ((1u << lane) - 1u))] =
-                            (static_cast<uint32_t>(row) << 4) | (absent_list << 3) | static_cast<uint32_t>(q);
-                    queued += __popc(m);
-                    __syncwarp();
-                    if (queued >= 32) {
-                        queued -= 32;
-                        const uint32_t e = queue[queued + lane];
-                        __syncwarp();
-                        resolve(e);
+                    if (q < n_valid) {
+                        uint32_t mn;
+                        if constexpr (B == 1) mn = acc[0] & 0xffffu;
+                        else mn = (acc[q >> 1] >> ((q & 1) * 16)) & 0xffffu;
+                        if (valid) {
+                            // (mn >= n: a rank row with a hole, i.e. not a permutation -- counted nowhere, reported by the host calls)
+                            if (mn == 0) zero |= 1u << ((q >> 1) + (q & 1) * 16);
+                            else if (mn < static_cast<uint32_t>(n)) hist_add<P16>(list_hist + q * work.hist_stride, side + static_cast<int>(mn), 1u);
+                        }
                     }
                 }
+                // min == 0: the wanted statistic is the mex; queue (row, permutation), resolve 32 at a time
+                if (__any_sync(FULL_MASK, zero != 0)) queue_events(zero, (static_cast<uint32_t>(row) << 4) | (absent_list << 3));
             }
 #pragma unroll
             for (int i = 0; i < REGS; ++i) acc[i] = 0xffffffffu;
@@ -636,13 +658,21 @@ list_kernel(const pgx_plan plan, const uint16_t *__restrict__ perms, const long 
 
     if constexpr (P16) {
         if (minima) {
-            // ---- count the item's scratch minima in B packed pan-side histograms where the table was ----
-            uint32_t *s_hist = reinterpret_cast<uint32_t *>(table);            // [B][words]; pan bin k: half (k & 1) of word k >> 1
-            const int words = (n + 1) >> 1;
-            for (int i = tid; i < (B * words + 3) >> 2; i += blockDim.x)
+            // ---- count the item's scratch minima in packed pan-side histograms where the table was ----
+            // B >= 2: plane i counts permutation 2i in the low and 2i + 1 in the high half of word i * plane + k (pan bin
+            // k), so both halves of a packed minimum register are counted with a constant increment.  B == 1: bin k in
+            // half k & 1 of word k >> 1.  A minimum is clamped to n first: bin 0 (min 0, the mex events) and bin n (no
+            // permutation of the batch, or a rank row with a hole) are counted but never flushed.  Bin 0 counts rows
+            // holding the rank-0 genome and cannot exceed its gene count; carries out of bin n only reach bin n of the
+            // other half or leave the word.
+            uint32_t *s_hist = reinterpret_cast<uint32_t *>(table);
+            const int plane = (n + 2) & ~1;
+            const int s_words = B == 1 ? (n + 2) >> 1 : REGS * plane;
+            for (int i = tid; i < (s_words + 3) >> 2; i += blockDim.x)
                 reinterpret_cast<uint4 *>(s_hist)[i] = make_uint4(0u, 0u, 0u, 0u);
             __syncthreads();
             const uint16_t *__restrict__ slot = minima + static_cast<size_t>(blockIdx.x) * plan.n_rows * B;
+            const uint32_t clamp = static_cast<uint32_t>(n) * 0x10001u;
             constexpr int AHEAD = 4;                      // rows per lane in flight: the scratch comes back from HBM
             for (long long t = tid >> 5;; t += blockDim.x >> 5) {
                 const long long task = t * splits + split;
@@ -663,22 +693,41 @@ list_kernel(const pgx_plan plan, const uint16_t *__restrict__ perms, const long 
                     }
 #pragma unroll
                     for (int j = 0; j < AHEAD; ++j) {
+                        if (r0 + 32 * j >= d.w) continue;
 #pragma unroll
-                        for (int q = 0; q < B; ++q) {
-                            const uint32_t mn = B == 1 ? v[j][0] & 0xffffu : (v[j][q >> 1] >> ((q & 1) * 16)) & 0xffffu;
-                            // pan bins 1 .. N-1 only: 0 went to the mex queue, >= N is a rank row with a hole
-                            if (q < n_valid && mn - 1u < static_cast<uint32_t>(n - 1))
-                                atomicAdd(s_hist + q * words + (mn >> 1), 1u << ((mn & 1) * 16));
+                        for (int i = 0; i < REGS; ++i) {
+                            const uint32_t c = __vminu2(v[j][i], clamp);
+                            if constexpr (B == 1) {
+                                atomicAdd(s_hist + (c >> 1), 1u << ((c & 1u) * 16));
+                            } else {
+                                atomicAdd(s_hist + i * plane + (c & 0xffffu), 1u);
+                                atomicAdd(s_hist + i * plane + (c >> 16), 0x10000u);
+                            }
                         }
                     }
                 }
             }
             __syncthreads();
-            for (int q = 0; q < n_valid; ++q) {
-                uint32_t *dst = work.hist + (p0 + q) * work.hist_stride;
+            // global word w holds pan bins 2w and 2w + 1; bin n (odd n: the high half of the last word) is core bin 0
+            const int words = (n + 1) >> 1;
+            for (int i = 0; i < REGS && 2 * i < n_valid; ++i) {
+                uint32_t *dst0 = work.hist + (p0 + 2 * i) * work.hist_stride;
                 for (int w = tid; w < words; w += blockDim.x) {
-                    const uint32_t c = s_hist[q * words + w];
-                    if (c) atomicAdd(dst + w, c);
+                    uint32_t lo, hi;                      // global word w (pan bins 2w, 2w + 1) of permutations 2i and 2i + 1
+                    if constexpr (B == 1) {
+                        lo = s_hist[w];
+                    } else {
+                        const uint2 c = *reinterpret_cast<const uint2 *>(s_hist + i * plane + 2 * w);
+                        lo = __byte_perm(c.x, c.y, 0x5410);
+                        hi = __byte_perm(c.x, c.y, 0x7632);
+                    }
+                    const uint32_t keep = (w == 0 ? 0xffff0000u : 0xffffffffu) & (2 * w + 1 == n ? 0x0000ffffu : 0xffffffffu);
+                    lo &= keep;
+                    if (lo) atomicAdd(dst0 + w, lo);
+                    if constexpr (B > 1) {
+                        hi &= keep;
+                        if (2 * i + 1 < n_valid && hi) atomicAdd(dst0 + work.hist_stride + w, hi);
+                    }
                 }
             }
             __syncthreads();                              // the next item's table overwrites the histograms
