@@ -349,6 +349,35 @@ int pgx_random_perms(uint64_t seed, int64_t first, int64_t n_perm, int32_t n_gen
 int pgx_curve_moments(const int32_t *d_curves, int64_t n_rows, int64_t width, int64_t *d_sum, uint64_t *d_sumsq,
                       int32_t *d_min, int32_t *d_max, int32_t accumulate, void *stream);
 
+/* Shared-gene matrix S = X^T X of a planned table: S[k][l] = genes present in both genome k and genome l, S[k][k] =
+ * d_colsum[k].  With A the absent-list rows, u[k] the absent-list rows listing genome k and n_full the universal genes,
+ * for k != l the plan's classes contribute
+ *
+ *   S[k][l] = n_full + sum(w_absent) - w_absent[k] - w_absent[l]            universal and single-absence genes
+ *           + |A| - u[k] - u[l] + #{absent-list rows listing k and l}       absent lists
+ *           + #{present-list rows listing k and l}                          present lists
+ *           + sum over bitmap rows of bit_k * bit_l                         bitmap rows: an 8-bit integer GEMM
+ *
+ * (empty and single-presence genes add nothing off the diagonal).  n_full is derived on the device from genome 0's
+ * diagonal; a plan whose rows and vectors do not add up to d_colsum[0] fails with PGX_ERR_INVALID.  The bitmap rows are
+ * expanded, a K-slab at a time, into a genome-major 0 / 1 byte matrix E [N][K_slab] in the workspace and S += E E^T
+ * runs on the tensor cores (tcgen05.mma kind::i8, s32 accumulators), upper-triangle tiles only; the upper triangle is
+ * then mirrored into the lower one.  oracle/shared_np.py restates all of it.
+ *   d_shared   : [N][N] int32, 16-byte aligned; overwritten
+ *   d_work     : caller workspace of work_bytes >= N * 128 bytes, 16-byte aligned; the slab width K_slab is the
+ *                largest multiple of 128 with N * K_slab <= work_bytes (capped at the bitmap rows), so a smaller
+ *                workspace only means more slabs
+ * Asynchronous on ``stream`` except for one wait, after the small kernels that derive n_full, to check the plan. */
+int pgx_shared_genes(const pgx_plan *plan, int32_t *d_shared, void *d_work, int64_t work_bytes, void *stream);
+
+/* Row sums of the genomic-fluidity distances (Kislyuk et al., BMC Genomics 12:32, 2011) of a shared-gene matrix:
+ *   d_row_sums[k] = sum over l != k of d_kl,   d_kl = (M_k + M_l - 2 S[k][l]) / (M_k + M_l),   M = diag(S)
+ * in float64 (a pair with M_k + M_l = 0 gives NaN).  Fixed reduction order: two calls give the same bits.  Fluidity
+ * is sum(d_row_sums) / 2 over N (N - 1) / 2 pairs.
+ *   d_shared : [N][N] int32 as pgx_shared_genes writes it, 4-byte aligned;  d_row_sums : [N] float64, 8-byte aligned
+ * 1 <= N <= 65503.  Asynchronous on ``stream``. */
+int pgx_fluidity_rows(const int32_t *d_shared, int32_t n_genomes, double *d_row_sums, void *stream);
+
 #ifdef __cplusplus
 }
 #endif

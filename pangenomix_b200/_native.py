@@ -23,7 +23,7 @@ EXPORTS = (
     "pgx_expand_deltas", "pgx_host_plan_create", "pgx_host_plan_destroy", "pgx_plan_create", "pgx_plan_upload",
     "pgx_plan_destroy", "pgx_set_trace", "pgx_legacy_random_raw", "pgx_coo_marginals", "pgx_frequency_spectrum",
     "pgx_coo_marginals_host", "pgx_ks_scratch_bytes", "pgx_ks_montecarlo", "pgx_ks_montecarlo_host", "pgx_expand_split", "pgx_split_head",
-    "pgx_random_perms", "pgx_curve_moments",
+    "pgx_random_perms", "pgx_curve_moments", "pgx_shared_genes", "pgx_fluidity_rows",
 )
 
 
@@ -178,6 +178,10 @@ def load():
     lib.pgx_random_perms.argtypes = [ctypes.c_uint64, i64, i64, i32, vp, vp]
     lib.pgx_curve_moments.restype = ctypes.c_int
     lib.pgx_curve_moments.argtypes = [vp, i64, i64, vp, vp, vp, vp, i32, vp]
+    lib.pgx_shared_genes.restype = ctypes.c_int
+    lib.pgx_shared_genes.argtypes = [plan_p, vp, vp, i64, vp]
+    lib.pgx_fluidity_rows.restype = ctypes.c_int
+    lib.pgx_fluidity_rows.argtypes = [vp, i32, vp, vp]
     lib.pgx_profile_enable.restype = ctypes.c_int
     lib.pgx_profile_enable.argtypes = [i32]
     lib.pgx_profile_read.restype = ctypes.c_int

@@ -12,7 +12,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 REPO = os.path.dirname(HERE)
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libpgx_b200.so")
-SOURCES = ["pgx_api.cu", "pgx_rarefy.cu", "pgx_bernoulli.cu", "pgx_heaps.cu", "pgx_betabin.cu", "pgx_perm.cu"]
+SOURCES = ["pgx_api.cu", "pgx_rarefy.cu", "pgx_bernoulli.cu", "pgx_heaps.cu", "pgx_betabin.cu", "pgx_perm.cu", "pgx_shared.cu"]
 HOST_SOURCES = ["pgx_rng.cpp", "pgx_plan.cpp", "pgx_inflate.cpp", "pgx_expand.cpp", "pgx_plan_build.cpp"]            # plain C++ (g++): AVX2 paths are selected at run time
 HEADERS = [os.path.join(CSRC, "pgx_common.cuh"), os.path.join(REPO, "include", "pgx.h")]
 

@@ -293,6 +293,48 @@ class PanCoreEngine:
         return CurveMoments(int(num_iter), s.cpu().numpy(), q.cpu().numpy().view(np.uint64), lo.cpu().numpy(),
                             hi.cpu().numpy())
 
+    # ---- genome x genome comparisons -------------------------------------------------------
+    def shared_workspace_bytes(self):
+        """Workspace of pgx_shared_genes: the whole bitmap expanded as one K-slab, at most SHARED_WORK_CAP bytes (a
+        larger table takes several slabs), at least the N x 128 bytes the call needs."""
+        hp, n = self.host_plan, self.n_genomes
+        k_total = hp.n_superblocks * 1024 * hp.slice_words if hp.n_long else 0
+        return max(128 * n, min(n * k_total, SHARED_WORK_CAP))
+
+    def shared_genes_device(self, out=None):
+        """Shared-gene matrix S = X^T X of the table (pgx_shared_genes): a CUDA int32 tensor [N, N] with S[k, l] =
+        genes present in both genome k and genome l.  The workspace is a torch allocation, released on return.
+        Asynchronous on the current torch stream after a short wait in which the library checks the plan."""
+        torch = _torch()
+        n = self.n_genomes
+        if out is None:
+            out = torch.empty((n, n), dtype=torch.int32, device=self.device)
+        elif out.shape != (n, n) or out.dtype != torch.int32 or not out.is_contiguous() or out.device != self.device:
+            raise ValueError("out must be a contiguous int32 [N, N] tensor on the engine's device")
+        work_bytes = self.shared_workspace_bytes()
+        with torch.cuda.device(self.device):
+            work = torch.empty(work_bytes, dtype=torch.uint8, device=self.device)
+            _native.check(self.lib.pgx_shared_genes(ctypes.byref(self.c_plan), out.data_ptr(), work.data_ptr(),
+                                                    work_bytes, torch.cuda.current_stream(self.device).cuda_stream))
+        return out
+
+    def fluidity_rows_device(self, shared):
+        """R[k] = sum over l != k of the fluidity distances d_kl of a shared-gene matrix (pgx_fluidity_rows) as a
+        CUDA float64 tensor [N].  Asynchronous on the current torch stream."""
+        torch = _torch()
+        n = self.n_genomes
+        if shared.shape != (n, n) or shared.dtype != torch.int32 or not shared.is_contiguous() or \
+                shared.device != self.device:
+            raise ValueError("shared must be a contiguous int32 [N, N] tensor on the engine's device")
+        rows = torch.empty(n, dtype=torch.float64, device=self.device)
+        with torch.cuda.device(self.device):
+            _native.check(self.lib.pgx_fluidity_rows(shared.data_ptr(), n, rows.data_ptr(),
+                                                     torch.cuda.current_stream(self.device).cuda_stream))
+        return rows
+
+
+SHARED_WORK_CAP = 4 << 30          # bytes of expanded bitmap rows per slab of pgx_shared_genes
+
 
 def fit_heaps_device(curves, n_points=None):
     """Heaps-law fits of every row of a CUDA tensor of curves (int32 or float64, contiguous rows).

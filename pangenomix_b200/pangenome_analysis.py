@@ -13,13 +13,15 @@ reference; the work is done by libpgx_b200 on a B200:
   simulation on the GPU (pgx_ks_montecarlo_host), consuming the global numpy RNG exactly as ``np.random.choice`` does
 
 Extension beside the drop-in: ``estimate_pan_core_summary`` -- mean / std / min / max of the pan/core curves over
-genome orders drawn on the GPU from a seeded counter-based stream (not numpy's), reduced on the GPU.
+genome orders drawn on the GPU from a seeded counter-based stream (not numpy's), reduced on the GPU;
+``shared_gene_counts`` (genome x genome shared genes, X^T X on the tensor cores) and ``compute_genomic_fluidity``.
 
 Not provided (out of scope, SURVEY.md section 2): the coordinate-descent variant the
 reference marks "DON'T USE THIS" and the mlst wrapper.
 """
 from __future__ import print_function
 
+import math
 import weakref
 
 import collections
@@ -211,6 +213,66 @@ def summary_frame(moments, num_strains):
     data = np.vstack([mean, std, np.asarray(moments.min, dtype=np.float64), np.asarray(moments.max, dtype=np.float64)])
     return pd.DataFrame(data, index=['mean', 'std', 'min', 'max'], columns=_labels(('Pan', 'Core'), num_strains),
                         copy=False)
+
+
+def shared_gene_counts(df_genes, device=None):
+    '''
+    Genome x genome shared-gene matrix S = X^T X of a binary gene x genome table: S[k, l] is the number of genes
+    present in both genome k and genome l, S[k, k] the genes of genome k.  The start of clustering genomes by gene
+    content, Jaccard distances and genomic fluidity.  Computed on the GPU from the table's plan (shared with
+    estimate_pan_core_size / estimate_pan_core_summary, so the table is not planned again), the dense part as an
+    8-bit integer matrix product on the tensor cores.  Prints nothing and leaves ``np.random`` untouched.
+
+    Returns
+    -------
+    df_shared : pd.DataFrame
+        int32, N x N, index and columns ``df_genes.columns``.
+    '''
+    engine = _engine_for(df_genes, device)
+    shared = engine.shared_genes_device().cpu().numpy()
+    return pd.DataFrame(shared, index=df_genes.columns, columns=df_genes.columns, copy=False)
+
+
+def compute_genomic_fluidity(df_genes, device=None):
+    '''
+    Genomic fluidity (Kislyuk, Haegeman, Bergman & Weitz, BMC Genomics 12:32, 2011): the mean over genome pairs of
+    the share of their genes that the two genomes do not share, (|U_k| + |U_l|) / (M_k + M_l) with U the genes of one
+    genome absent from the other and M the genomes' gene counts.  Unlike Heaps' alpha from rarefaction it does not
+    depend on the order genomes were sampled in.  Its standard error is the leave-one-genome-out jackknife.
+
+    The shared-gene matrix and the per-genome sums of the pair distances are computed on the GPU (see
+    shared_gene_counts); only N numbers come back to the host.  Prints nothing and leaves ``np.random`` untouched.
+
+    Returns
+    -------
+    pd.Series
+        float64 entries ``fluidity``, ``jackknife_se`` (NaN for two genomes) and ``n_genomes``.  Tables of fewer
+        than two genomes raise ValueError.
+    '''
+    _, num_strains = df_genes.shape
+    if num_strains < 2:
+        raise ValueError("genomic fluidity needs at least two genomes, got %d" % num_strains)
+    engine = _engine_for(df_genes, device)
+    rows = engine.fluidity_rows_device(engine.shared_genes_device()).cpu().numpy()
+    return fluidity_series(rows)
+
+
+def fluidity_series(row_sums):
+    """The Series of compute_genomic_fluidity() from R[k] = sum over l != k of the pair distances d_kl:
+    T = fsum(R) / 2 is the sum over pairs, fluidity = T / C(N, 2), leave-one-genome-out values
+    (T - R[i]) / C(N - 1, 2) and jackknife_se = sqrt((N - 1) / N * sum((phi_i - mean phi)^2))."""
+    rows = np.asarray(row_sums, dtype=np.float64)
+    n = int(rows.shape[0])
+    if n < 2:
+        raise ValueError("genomic fluidity needs at least two genomes, got %d" % n)
+    total = math.fsum(rows) / 2
+    fluidity = total / (n * (n - 1) / 2)
+    if n > 2:
+        loo = (total - rows) / ((n - 1) * (n - 2) / 2)
+        se = math.sqrt((n - 1) / n * float(np.sum((loo - loo.mean()) ** 2)))
+    else:
+        se = np.nan
+    return pd.Series({'fluidity': fluidity, 'jackknife_se': se, 'n_genomes': float(n)}, dtype=np.float64)
 
 
 def compute_bernoulli_grid_core_genome(df_genes_dense,
