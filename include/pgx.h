@@ -378,6 +378,71 @@ int pgx_shared_genes(const pgx_plan *plan, int32_t *d_shared, void *d_work, int6
  * 1 <= N <= 65503.  Asynchronous on ``stream``. */
 int pgx_fluidity_rows(const int32_t *d_shared, int32_t n_genomes, double *d_row_sums, void *stream);
 
+/* Exact pan/core rarefaction: the mean and variance of the pan and core sizes of the first k genomes over ALL genome
+ * orders, without sampling.  The first k genomes of a uniformly random order are a uniformly random k-subset T; with
+ * m_g the genomes holding gene g, s_gh the genomes holding both g and h, a_gh = N - m_g - m_h + s_gh the genomes
+ * lacking both, and rho(v, k) = C(v, k) / C(N, k) (the chance that T lies inside a given set of v genomes):
+ *
+ *   E[core_k] = sum_g rho(m_g, k)                    Var[core_k] = E[core_k] + 2 sum_{g<h} rho(s_gh, k) - E[core_k]^2
+ *   E[pan_k]  = G - sum_g rho(N - m_g, k)  (Mao's tau; Colwell, Mao & Chang, Ecology 85:2717, 2004)
+ *   Var[pan_k] = Z_k + 2 sum_{g<h} rho(a_gh, k) - Z_k^2,   Z_k = sum_g rho(N - m_g, k)
+ *
+ * The variance is conditional on the table (the spread over orders of these N genomes, what the permutation std
+ * converges to).  The means need the spectrum of m; the variances the pair histograms
+ * H_s[v] = #{g < h : s_gh = v} and H_a[v] = #{g < h : a_gh = v}.
+ *
+ * Gene-frequency spectrum of a planned table: d_spectrum[v] (int64 [N + 1]) = genes present in exactly v genomes,
+ * counted from the plan alone (rows by their lists or bit counts, the closed-form classes from the per-genome vectors;
+ * the universal and empty counts are derived on the device).  A plan whose rows and vectors do not add up to whole
+ * universal and empty counts fails with PGX_ERR_INVALID.  Asynchronous on ``stream`` except for one final wait that
+ * checks the plan. */
+int pgx_plan_spectrum(const pgx_plan *plan, int64_t *d_spectrum, void *stream);
+
+/* Pair overlap histograms H_s and H_a (int64 [N + 1] each, 8-byte aligned; overwritten) over the unordered pairs of
+ * distinct genes of the whole table, closed-form genes included.  With e / u the empty / universal genes,
+ * p1 = sum(w_present), a1 = sum(w_absent), and for a stored (list or bitmap) row h: m_h, Wp_h = sum of w_present
+ * and Wa_h = sum of w_absent over the genomes holding h, the pairs count as follows ((s, a): count):
+ *
+ *   empty x row h            (0, N - m_h): e
+ *   universal x row h        (m_h, 0): u
+ *   single-genome x row h    (1, N - m_h): Wp_h          (0, N - 1 - m_h): p1 - Wp_h
+ *   single-absence x row h   (m_h - 1, 0): Wa_h          (m_h, 1): a1 - Wa_h
+ *   empty x empty / universal / single-genome / single-absence   (0, N): C(e, 2)  (0, 0): e u  (0, N - 1): e p1
+ *                                                                (0, 1): e a1
+ *   universal x universal / single-genome / single-absence       (N, 0): C(u, 2)  (1, 0): u p1  (N - 1, 0): u a1
+ *   single-genome x single-genome, same / other genome           (1, N - 1): sum_c C(wp_c, 2)  (0, N - 2): the rest
+ *   single-absence x single-absence, same / other genome         (N - 1, 1): sum_c C(wa_c, 2)  (N - 2, 0): the rest
+ *   single-genome x single-absence, same / other genome          (0, 0): sum_c wp_c wa_c       (1, 1): the rest
+ *   row x row                s from an 8-bit integer GEMM, a = N - m_g - m_h + s
+ *
+ * The stored rows are sorted by m (a tile of sorted rows then knows the range of its s and a), expanded in panels
+ * into a gene-major 0 / 1 byte matrix E [P][N_pad] (N_pad = N rounded up to 128) and E E^T runs over panel pairs
+ * I <= J on the tensor cores (tcgen05.mma kind::i8, s32 accumulators; the GEMM of pgx_shared_genes with a histogram
+ * epilogue): a tile counts into shared-memory bins when its value range fits them, else into the global bins.
+ * oracle/exact_np.py restates all of it.
+ *   d_work     : caller workspace, 256-byte aligned, of work_bytes >= pgx_pair_overlap_work_bytes(N, R, 0) bytes,
+ *                R = n_rows + n_long (the rows' bookkeeping plus two panels of 256 E rows, or all R rows when fewer);
+ *                pgx_pair_overlap_work_bytes(N, R, 1) holds every E row in one panel, and any size in between works
+ *                with more panels
+ * The plan is checked as by pgx_plan_spectrum.  Asynchronous on ``stream`` except for that one wait. */
+int pgx_pair_overlap_histograms(const pgx_plan *plan, int64_t *d_hist_shared, int64_t *d_hist_absent, void *d_work,
+                                int64_t work_bytes, void *stream);
+
+/* Workspace bytes of pgx_pair_overlap_histograms for N genomes and R = n_rows + n_long stored rows: the minimum
+ * (one_panel == 0) or the size that holds every stored row in one panel (one_panel != 0).  0 for N outside
+ * 1 .. 65503 or R outside 0 .. 2^31 - 513. */
+int64_t pgx_pair_overlap_work_bytes(int32_t n_genomes, int64_t n_stored_rows, int32_t one_panel);
+
+/* The four exact curves from the spectrum and the pair histograms: d_out [4][N] float64 (8-byte aligned), rows
+ * E[pan_k], Var[pan_k], E[core_k], Var[core_k] for k = 1 .. N.  One thread per k sums w[v] rho(v, k) over
+ * v = N .. k with rho(N, k) = 1 and rho(v - 1, k) = rho(v, k) (v - k) / v (products, never lgamma differences, which
+ * lose about 1e-10 relative at N = 50,000; an underflow to 0 ends the sum), in that fixed order: two calls give the
+ * same bits, and rho(v, N) = [v = N] makes both variances exactly 0 at k = N.  With both histograms null only the
+ * two mean rows are written.  n_genes is G (the table's genes, closed-form ones included).  1 <= N <= 65503.
+ * Asynchronous on ``stream``. */
+int pgx_rarefaction_moments(const int64_t *d_spectrum, const int64_t *d_hist_shared, const int64_t *d_hist_absent,
+                            int64_t n_genes, int32_t n_genomes, double *d_out, void *stream);
+
 #ifdef __cplusplus
 }
 #endif

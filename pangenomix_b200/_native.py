@@ -24,6 +24,7 @@ EXPORTS = (
     "pgx_plan_destroy", "pgx_set_trace", "pgx_legacy_random_raw", "pgx_coo_marginals", "pgx_frequency_spectrum",
     "pgx_coo_marginals_host", "pgx_ks_scratch_bytes", "pgx_ks_montecarlo", "pgx_ks_montecarlo_host", "pgx_expand_split", "pgx_split_head",
     "pgx_random_perms", "pgx_curve_moments", "pgx_shared_genes", "pgx_fluidity_rows",
+    "pgx_plan_spectrum", "pgx_pair_overlap_histograms", "pgx_pair_overlap_work_bytes", "pgx_rarefaction_moments",
 )
 
 
@@ -182,6 +183,14 @@ def load():
     lib.pgx_shared_genes.argtypes = [plan_p, vp, vp, i64, vp]
     lib.pgx_fluidity_rows.restype = ctypes.c_int
     lib.pgx_fluidity_rows.argtypes = [vp, i32, vp, vp]
+    lib.pgx_plan_spectrum.restype = ctypes.c_int
+    lib.pgx_plan_spectrum.argtypes = [plan_p, vp, vp]
+    lib.pgx_pair_overlap_histograms.restype = ctypes.c_int
+    lib.pgx_pair_overlap_histograms.argtypes = [plan_p, vp, vp, vp, i64, vp]
+    lib.pgx_pair_overlap_work_bytes.restype = i64
+    lib.pgx_pair_overlap_work_bytes.argtypes = [i32, i64, i32]
+    lib.pgx_rarefaction_moments.restype = ctypes.c_int
+    lib.pgx_rarefaction_moments.argtypes = [vp, vp, vp, i64, i32, vp, vp]
     lib.pgx_profile_enable.restype = ctypes.c_int
     lib.pgx_profile_enable.argtypes = [i32]
     lib.pgx_profile_read.restype = ctypes.c_int

@@ -1,5 +1,7 @@
-// Genome x genome shared-gene matrix S = X^T X of a planned table (pgx_shared_genes) and the per-genome sums of
-// genomic-fluidity distances (pgx_fluidity_rows).  The decomposition of S over the plan's gene classes is stated in
+// Genome x genome shared-gene matrix S = X^T X of a planned table (pgx_shared_genes), the per-genome sums of
+// genomic-fluidity distances (pgx_fluidity_rows), and the gene-pair overlap histograms and exact rarefaction moments
+// further down (pgx_plan_spectrum, pgx_pair_overlap_histograms, pgx_rarefaction_moments), whose GEMM shares the
+// mainloop of S.  The decomposition of S over the plan's gene classes is stated in
 // include/pgx.h; oracle/shared_np.py restates it in numpy.
 //
 //   count   u[k] / p[k] = absent / present list rows listing genome k, |A|, sum(w_absent) and the bitmap popcount
@@ -223,10 +225,12 @@ __host__ __device__ inline int64_t group_tiles(int32_t g, int32_t col_tiles)
     return int64_t(col_tiles - g * (GROUP_ROWS / 2)) * GROUP_ROWS;
 }
 
-// one CTA per tile of the order above; a tile without an entry above the diagonal (cb < rb / 2) returns at once
-__global__ void __launch_bounds__(GEMM_THREADS, 1) shared_gemm_kernel(const __grid_constant__ CUtensorMap map,
-                                                                       int32_t n, int32_t k_blocks,
-                                                                       int32_t *__restrict__ shared)
+// One CTA per tile of the order above over the rows 0 .. n - 1 of the operand ``map`` describes, E E^T on tcgen05.
+// A tile without an entry above the diagonal (cb < rb / 2), or one the epilogue skips, returns at once.  The epilogue
+// reads the tile's accumulator from tensor memory: Epi::skip(rb, cb) and Epi::run(tmem, warp, lane, m0, n0, n, stages),
+// where ``stages`` (the shared-memory stage buffers, free once the MMAs are done) is its scratch.
+template <class Epi>
+__device__ __forceinline__ void gemm_tiles(const CUtensorMap &map, int32_t n, int32_t k_blocks, const Epi &epi)
 {
     const int32_t row_tiles = (n + BM - 1) / BM, col_tiles = (n + BN - 1) / BN;
     int64_t id = blockIdx.x;
@@ -234,7 +238,7 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) shared_gemm_kernel(const __gr
     while (id >= group_tiles(g, col_tiles)) id -= group_tiles(g++, col_tiles);
     const int32_t cb = g * (GROUP_ROWS / 2) + static_cast<int32_t>(id / GROUP_ROWS);
     const int32_t rb = g * GROUP_ROWS + static_cast<int32_t>(id % GROUP_ROWS);
-    if (rb >= row_tiles || cb < rb / 2) return;
+    if (rb >= row_tiles || cb < rb / 2 || epi.skip(rb, cb)) return;
     extern __shared__ uint8_t smem_raw[];
     __shared__ __align__(8) uint64_t full_bar[STAGES], empty_bar[STAGES], done_bar;
     __shared__ uint32_t tmem_base;
@@ -286,43 +290,63 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) shared_gemm_kernel(const __gr
     }
     __syncwarp();
 
-    // epilogue: warp w owns TMEM lanes 32 w .. 32 w + 31 = tile rows; thread = one row, 32 columns per load
+    // epilogue: warp w owns TMEM lanes 32 w .. 32 w + 31 = tile rows; thread = one row
     mbar_wait(smem_u32(&done_bar), 0);
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    const int32_t row = m0 + 32 * warp + lane;
-    int32_t *dst = shared + static_cast<int64_t>(row) * n;
-    const bool vec = (n & 3) == 0;
-#pragma unroll 1
-    for (int c = 0; c < BN; c += 32) {
-        uint32_t acc[32];
-        tmem_ld_32(tmem + (static_cast<uint32_t>(32 * warp) << 16) + c, acc);
-        const int32_t col0 = n0 + c;
-        if (row >= n || col0 + 31 <= row || col0 >= n) continue;
-        if (vec && col0 > row && col0 + 32 <= n) {
-            int4 *p = reinterpret_cast<int4 *>(dst + col0);
-#pragma unroll
-            for (int q = 0; q < 8; ++q) {
-                int4 v = p[q];
-                v.x += static_cast<int32_t>(acc[4 * q]);
-                v.y += static_cast<int32_t>(acc[4 * q + 1]);
-                v.z += static_cast<int32_t>(acc[4 * q + 2]);
-                v.w += static_cast<int32_t>(acc[4 * q + 3]);
-                p[q] = v;
-            }
-        } else {
-#pragma unroll
-            for (int q = 0; q < 32; ++q) {
-                const int32_t col = col0 + q;
-                if (col > row && col < n) dst[col] += static_cast<int32_t>(acc[q]);
-            }
-        }
-    }
+    epi.run(tmem, warp, lane, m0, n0, n, stages);
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
     if (warp == 2) {
         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
         asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(TMEM_COLS) : "memory");
     }
+}
+
+// S epilogue: the tile, 32 columns per load, added into S above the diagonal
+struct SharedEpilogue {
+    int32_t *shared;
+
+    __device__ __forceinline__ bool skip(int32_t, int32_t) const { return false; }
+
+    __device__ __forceinline__ void run(uint32_t tmem, int warp, int lane, int32_t m0, int32_t n0, int32_t n,
+                                        uint32_t) const
+    {
+        const int32_t row = m0 + 32 * warp + lane;
+        int32_t *dst = shared + static_cast<int64_t>(row) * n;
+        const bool vec = (n & 3) == 0;
+#pragma unroll 1
+        for (int c = 0; c < BN; c += 32) {
+            uint32_t acc[32];
+            tmem_ld_32(tmem + (static_cast<uint32_t>(32 * warp) << 16) + c, acc);
+            const int32_t col0 = n0 + c;
+            if (row >= n || col0 + 31 <= row || col0 >= n) continue;
+            if (vec && col0 > row && col0 + 32 <= n) {
+                int4 *p = reinterpret_cast<int4 *>(dst + col0);
+#pragma unroll
+                for (int q = 0; q < 8; ++q) {
+                    int4 v = p[q];
+                    v.x += static_cast<int32_t>(acc[4 * q]);
+                    v.y += static_cast<int32_t>(acc[4 * q + 1]);
+                    v.z += static_cast<int32_t>(acc[4 * q + 2]);
+                    v.w += static_cast<int32_t>(acc[4 * q + 3]);
+                    p[q] = v;
+                }
+            } else {
+#pragma unroll
+                for (int q = 0; q < 32; ++q) {
+                    const int32_t col = col0 + q;
+                    if (col > row && col < n) dst[col] += static_cast<int32_t>(acc[q]);
+                }
+            }
+        }
+    }
+};
+
+__global__ void __launch_bounds__(GEMM_THREADS, 1) shared_gemm_kernel(const __grid_constant__ CUtensorMap map,
+                                                                       int32_t n, int32_t k_blocks,
+                                                                       int32_t *__restrict__ shared)
+{
+    gemm_tiles(map, n, k_blocks, SharedEpilogue{shared});
 }
 
 // ---- mirror -----------------------------------------------------------------------------------------------------
@@ -382,6 +406,548 @@ __global__ void __launch_bounds__(ROW_THREADS) fluidity_rows_kernel(const int32_
     if (threadIdx.x < ROWS && k0 + threadIdx.x < n) row_sums[k0 + threadIdx.x] = part[threadIdx.x][0];
 }
 
+// ---- pair overlap histograms and exact rarefaction moments ------------------------------------------------------
+// (pgx_plan_spectrum, pgx_pair_overlap_histograms, pgx_rarefaction_moments; the decomposition is stated in
+// include/pgx.h and restated in oracle/exact_np.py)
+//
+//   vectors  p1 = sum(w_present), a1 = sum(w_absent), nnz = sum(colsum) and the same-genome pair sums
+//   rows     m, Wp = sum of w_present over the row's genomes, Wa likewise, for every list and bitmap row; counted
+//            by m into rows_m / wp_m / wa_m
+//   classes  the universal count u = (nnz - sum of row m - p1 - a1 (N - 1)) / N and the empty count; a plan for
+//            which these are not whole and non-negative is refused
+//   closed   every pair with a closed-form gene, from the counts above, into H_s / H_a
+//   sort     the rows by m (counting sort), so that a GEMM tile knows the range its s and a can take
+//   expand   a panel of sorted rows into E [P][N_pad] (0 / 1 bytes, gene-major, genomes padded to 128)
+//   gemm     E E^T over panel pairs on the tensor cores with a histogram epilogue (gemm_tiles above)
+//   moments  T_w[k] = sum_v w[v] rho(v, k) for the four weight vectors, rho a running product
+struct ClassCounts {
+    int64_t p1, a1, nnz, sum_m, n_full, n_empty, same_p, same_a, same_pa;
+    int32_t valid, pad;
+};
+
+__device__ __forceinline__ void hist_add(unsigned long long *h, int64_t v, int64_t n, int64_t count)
+{
+    if (count != 0 && v >= 0 && v <= n) atomicAdd(h + v, static_cast<unsigned long long>(count));
+}
+
+// one warp per task (its rows share the list kind): m, Wp, Wa of every list row
+__global__ void pair_list_rows_kernel(const int32_t *__restrict__ tasks, int32_t n_tasks,
+                                      const uint16_t *__restrict__ sorted_idx, const int32_t *__restrict__ sorted_ptr,
+                                      const int32_t *__restrict__ w_present, const int32_t *__restrict__ w_absent,
+                                      int32_t n, const ClassCounts *__restrict__ cc, uint32_t *__restrict__ m_row,
+                                      unsigned long long *__restrict__ rows_m, unsigned long long *__restrict__ wp_m,
+                                      unsigned long long *__restrict__ wa_m)
+{
+    const int lane = threadIdx.x & 31;
+    const int32_t warp = static_cast<int32_t>((blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x) >> 5);
+    const int32_t n_warps = static_cast<int32_t>((gridDim.x * static_cast<int64_t>(blockDim.x)) >> 5);
+    for (int32_t t = warp; t < n_tasks; t += n_warps) {
+        const int4 task = reinterpret_cast<const int4 *>(tasks)[t];
+        const bool absent = (task.y >> 24) & 1;
+        for (int32_t r = task.z; r < task.z + task.w; ++r) {
+            const int32_t e0 = sorted_ptr[r], e1 = sorted_ptr[r + 1];
+            int32_t sp = 0, sa = 0;
+            for (int32_t e = e0 + lane; e < e1; e += 32) {
+                const int32_t c = sorted_idx[e];
+                sp += w_present[c];
+                sa += w_absent[c];
+            }
+            sp = __reduce_add_sync(0xffffffffu, sp);
+            sa = __reduce_add_sync(0xffffffffu, sa);
+            if (lane == 0) {
+                const int32_t m = absent ? n - (e1 - e0) : e1 - e0;
+                const int64_t wp = absent && wp_m ? cc->p1 - sp : sp, wa = absent && wp_m ? cc->a1 - sa : sa;
+                atomicAdd(rows_m + m, 1ull);
+                if (m_row) m_row[r] = static_cast<uint32_t>(m) | (absent ? 0x80000000u : 0u);
+                if (wp_m) {
+                    atomicAdd(wp_m + m, static_cast<unsigned long long>(wp));
+                    atomicAdd(wa_m + m, static_cast<unsigned long long>(wa));
+                }
+            }
+        }
+    }
+}
+
+// one block per 32 bitmap rows (one word of a superblock line): m, Wp, Wa by a masked sum over the genomes
+__global__ void __launch_bounds__(256) pair_bitmap_rows_kernel(const uint32_t *__restrict__ bits, int32_t n,
+                                                               int32_t slice_words, int32_t n_long, int32_t n_rows,
+                                                               const int32_t *__restrict__ w_present,
+                                                               const int32_t *__restrict__ w_absent,
+                                                               uint32_t *__restrict__ m_row,
+                                                               unsigned long long *__restrict__ rows_m,
+                                                               unsigned long long *__restrict__ wp_m,
+                                                               unsigned long long *__restrict__ wa_m)
+{
+    __shared__ int32_t part[3][32];
+    const int32_t line = 32 * slice_words;
+    const int32_t sb = blockIdx.x / line, w = blockIdx.x % line;
+    if (threadIdx.x < 32) part[0][threadIdx.x] = part[1][threadIdx.x] = part[2][threadIdx.x] = 0;
+    __syncthreads();
+    int32_t cnt[32], sp[32], sa[32];
+#pragma unroll
+    for (int b = 0; b < 32; ++b) cnt[b] = sp[b] = sa[b] = 0;
+    const bool sums = wp_m != nullptr;
+    for (int32_t c = threadIdx.x; c < n; c += blockDim.x) {
+        const uint32_t v = __ldg(&bits[(static_cast<int64_t>(sb) * n + c) * line + w]);
+        const int32_t p = sums ? w_present[c] : 0, a = sums ? w_absent[c] : 0;
+#pragma unroll
+        for (int b = 0; b < 32; ++b) {
+            const int32_t bit = (v >> b) & 1;
+            cnt[b] += bit;
+            sp[b] += bit * p;
+            sa[b] += bit * a;
+        }
+    }
+#pragma unroll
+    for (int b = 0; b < 32; ++b) {
+        const int32_t c = __reduce_add_sync(0xffffffffu, cnt[b]);
+        const int32_t p = __reduce_add_sync(0xffffffffu, sp[b]);
+        const int32_t a = __reduce_add_sync(0xffffffffu, sa[b]);
+        if ((threadIdx.x & 31) == 0) {
+            atomicAdd(&part[0][b], c);
+            atomicAdd(&part[1][b], p);
+            atomicAdd(&part[2][b], a);
+        }
+    }
+    __syncthreads();
+    if (threadIdx.x < 32) {
+        const int64_t k = static_cast<int64_t>(sb) * 1024 * slice_words + 32 * w + threadIdx.x;
+        if (k < n_long) {
+            const int32_t m = part[0][threadIdx.x];
+            atomicAdd(rows_m + m, 1ull);
+            if (m_row) m_row[n_rows + k] = static_cast<uint32_t>(m);
+            if (sums) {
+                atomicAdd(wp_m + m, static_cast<unsigned long long>(part[1][threadIdx.x]));
+                atomicAdd(wa_m + m, static_cast<unsigned long long>(part[2][threadIdx.x]));
+            }
+        }
+    }
+}
+
+// block-wide sums of Q int64 values per thread in a fixed order (blockDim.x = 1,024); the result in thread 0
+template <int Q>
+__device__ void block_sums(int64_t (&acc)[Q])
+{
+    __shared__ int64_t red[Q][32];
+    for (int q = 0; q < Q; ++q) {
+        for (int h = 16; h > 0; h >>= 1) acc[q] += __shfl_down_sync(0xffffffffu, acc[q], h);
+        if ((threadIdx.x & 31) == 0) red[q][threadIdx.x >> 5] = acc[q];
+    }
+    __syncthreads();
+    for (int q = 0; q < Q; ++q) {
+        acc[q] = 0;
+        for (int w = 0; w < 32; ++w) acc[q] += red[q][w];
+    }
+    __syncthreads();
+}
+
+// p1, a1, nnz and the same-genome pair sums of the per-genome vectors (one block of 1,024 threads)
+__device__ void vector_sums(int32_t n, const int32_t *__restrict__ colsum, const int32_t *__restrict__ w_present,
+                            const int32_t *__restrict__ w_absent, ClassCounts *cc)
+{
+    int64_t acc[6] = {0, 0, 0, 0, 0, 0};
+    for (int32_t c = threadIdx.x; c < n; c += blockDim.x) {
+        const int64_t p = w_present[c], a = w_absent[c];
+        acc[0] += p;
+        acc[1] += a;
+        acc[2] += colsum[c];
+        acc[3] += p * (p - 1) / 2;
+        acc[4] += a * (a - 1) / 2;
+        acc[5] += p * a;
+    }
+    block_sums(acc);
+    if (threadIdx.x == 0) {
+        cc->p1 = acc[0], cc->a1 = acc[1], cc->nnz = acc[2];
+        cc->same_p = acc[3], cc->same_a = acc[4], cc->same_pa = acc[5];
+    }
+    __syncthreads();
+}
+
+// universal and empty counts from the rows' spectrum: nnz = sum of row m + N u + p1 + (N - 1) a1
+__device__ void class_counts(int32_t n, int64_t n_genes, int64_t n_stored, const unsigned long long *__restrict__ rows_m,
+                             ClassCounts *cc)
+{
+    int64_t acc[1] = {0};
+    for (int32_t v = threadIdx.x; v <= n; v += blockDim.x) acc[0] += static_cast<int64_t>(rows_m[v]) * v;
+    block_sums(acc);
+    if (threadIdx.x == 0) {
+        cc->sum_m = acc[0];
+        const int64_t rest = cc->nnz - cc->sum_m - cc->p1 - cc->a1 * (n - 1);
+        cc->n_full = rest / n;
+        cc->n_empty = n_genes - cc->n_full - cc->p1 - cc->a1 - n_stored;
+        cc->valid = rest >= 0 && rest % n == 0 && cc->n_empty >= 0;
+    }
+    __syncthreads();
+}
+
+__global__ void __launch_bounds__(1024) pair_vectors_kernel(int32_t n, const int32_t *__restrict__ colsum,
+                                                            const int32_t *__restrict__ w_present,
+                                                            const int32_t *__restrict__ w_absent, ClassCounts *cc)
+{
+    vector_sums(n, colsum, w_present, w_absent, cc);
+}
+
+__global__ void __launch_bounds__(1024) pair_classes_kernel(int32_t n, int64_t n_genes, int64_t n_stored,
+                                                            const unsigned long long *__restrict__ rows_m,
+                                                            ClassCounts *cc)
+{
+    class_counts(n, n_genes, n_stored, rows_m, cc);
+}
+
+// the rows' spectrum (already in d_spectrum) + the closed-form classes; an inconsistent plan leaves -1 in bin 0
+__global__ void __launch_bounds__(1024) spectrum_finish_kernel(int32_t n, int64_t n_genes, int64_t n_stored,
+                                                               const int32_t *__restrict__ colsum,
+                                                               const int32_t *__restrict__ w_present,
+                                                               const int32_t *__restrict__ w_absent,
+                                                               int64_t *spectrum)
+{
+    __shared__ ClassCounts cc;
+    vector_sums(n, colsum, w_present, w_absent, &cc);
+    class_counts(n, n_genes, n_stored, reinterpret_cast<const unsigned long long *>(spectrum), &cc);
+    if (threadIdx.x == 0) {
+        if (!cc.valid) {
+            spectrum[0] = -1;
+            return;
+        }
+        spectrum[0] += cc.n_empty;
+        spectrum[n] += cc.n_full;
+        if (n > 1) {
+            spectrum[1] += cc.p1;
+            spectrum[n - 1] += cc.a1;
+        }
+    }
+}
+
+// every pair with a closed-form gene (the table in include/pgx.h): thread v = the rows with m = v; thread 0 also the
+// closed x closed pairs
+__global__ void pair_closed_kernel(int32_t n, const ClassCounts *__restrict__ ccp,
+                                   const unsigned long long *__restrict__ rows_m,
+                                   const unsigned long long *__restrict__ wp_m,
+                                   const unsigned long long *__restrict__ wa_m, unsigned long long *__restrict__ hs,
+                                   unsigned long long *__restrict__ ha)
+{
+    const ClassCounts cc = *ccp;
+    const int64_t e = cc.n_empty, u = cc.n_full, p1 = cc.p1, a1 = cc.a1;
+    const int32_t v = blockIdx.x * blockDim.x + threadIdx.x;
+    if (v == 0) {
+        hist_add(hs, 0, n, e * (e - 1) / 2), hist_add(ha, n, n, e * (e - 1) / 2);
+        hist_add(hs, 0, n, e * u), hist_add(ha, 0, n, e * u);
+        hist_add(hs, 0, n, e * p1), hist_add(ha, n - 1, n, e * p1);
+        hist_add(hs, 0, n, e * a1), hist_add(ha, 1, n, e * a1);
+        hist_add(hs, n, n, u * (u - 1) / 2), hist_add(ha, 0, n, u * (u - 1) / 2);
+        hist_add(hs, 1, n, u * p1), hist_add(ha, 0, n, u * p1);
+        hist_add(hs, n - 1, n, u * a1), hist_add(ha, 0, n, u * a1);
+        hist_add(hs, 1, n, cc.same_p), hist_add(ha, n - 1, n, cc.same_p);
+        hist_add(hs, 0, n, p1 * (p1 - 1) / 2 - cc.same_p), hist_add(ha, n - 2, n, p1 * (p1 - 1) / 2 - cc.same_p);
+        hist_add(hs, n - 1, n, cc.same_a), hist_add(ha, 1, n, cc.same_a);
+        hist_add(hs, n - 2, n, a1 * (a1 - 1) / 2 - cc.same_a), hist_add(ha, 0, n, a1 * (a1 - 1) / 2 - cc.same_a);
+        hist_add(hs, 0, n, cc.same_pa), hist_add(ha, 0, n, cc.same_pa);
+        hist_add(hs, 1, n, p1 * a1 - cc.same_pa), hist_add(ha, 1, n, p1 * a1 - cc.same_pa);
+    }
+    if (v > n) return;
+    const int64_t rows = static_cast<int64_t>(rows_m[v]);
+    if (rows == 0) return;
+    const int64_t wp = static_cast<int64_t>(wp_m[v]), wa = static_cast<int64_t>(wa_m[v]);
+    hist_add(hs, 0, n, e * rows), hist_add(ha, n - v, n, e * rows);
+    hist_add(hs, v, n, u * rows), hist_add(ha, 0, n, u * rows);
+    hist_add(hs, 1, n, wp), hist_add(ha, n - v, n, wp);
+    hist_add(hs, 0, n, p1 * rows - wp), hist_add(ha, n - 1 - v, n, p1 * rows - wp);
+    hist_add(hs, v - 1, n, wa), hist_add(ha, 0, n, wa);
+    hist_add(hs, v, n, a1 * rows - wa), hist_add(ha, 1, n, a1 * rows - wa);
+}
+
+// one block: cursor[v] = rows with m < v (exclusive scan of rows_m), in chunks of 1,024
+__global__ void __launch_bounds__(1024) pair_scan_kernel(int32_t n, const unsigned long long *__restrict__ rows_m,
+                                                         int32_t *__restrict__ cursor)
+{
+    __shared__ int32_t buf[1024];
+    __shared__ int32_t carry;
+    if (threadIdx.x == 0) carry = 0;
+    for (int32_t base = 0; base <= n; base += 1024) {
+        const int32_t v = base + threadIdx.x;
+        const int32_t x = v <= n ? static_cast<int32_t>(rows_m[v]) : 0;
+        buf[threadIdx.x] = x;
+        __syncthreads();
+        for (int h = 1; h < 1024; h <<= 1) {
+            const int32_t y = threadIdx.x >= h ? buf[threadIdx.x - h] : 0;
+            __syncthreads();
+            buf[threadIdx.x] += y;
+            __syncthreads();
+        }
+        if (v <= n) cursor[v] = carry + buf[threadIdx.x] - x;
+        __syncthreads();
+        if (threadIdx.x == 1023) carry += buf[1023];
+        __syncthreads();
+    }
+}
+
+// thread per row: its place in the m order (rows of equal m in any order: the histograms do not depend on it)
+__global__ void pair_sort_kernel(int32_t n_stored, const uint32_t *__restrict__ m_row, int32_t *__restrict__ cursor,
+                                 uint32_t *__restrict__ row_at, int32_t *__restrict__ m_sorted,
+                                 int32_t *__restrict__ pos_of)
+{
+    const int32_t r = blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= n_stored) return;
+    const uint32_t v = m_row[r];
+    const int32_t m = static_cast<int32_t>(v & 0x7fffffffu);
+    const int32_t p = atomicAdd(cursor + m, 1);
+    row_at[p] = static_cast<uint32_t>(r) | (v & 0x80000000u);
+    m_sorted[p] = m;
+    pos_of[r] = p;
+}
+
+// one warp per list row of the panel (sorted positions p0 .. p1 - 1): E row = the default byte, then the list's
+// genomes flipped
+__global__ void pair_expand_list_kernel(const uint32_t *__restrict__ row_at, int32_t p0, int32_t p1, int32_t n_rows,
+                                        const uint16_t *__restrict__ sorted_idx,
+                                        const int32_t *__restrict__ sorted_ptr, int32_t n, int32_t n_pad,
+                                        uint8_t *__restrict__ e)
+{
+    const int lane = threadIdx.x & 31;
+    const int32_t warp = static_cast<int32_t>((blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x) >> 5);
+    const int32_t n_warps = static_cast<int32_t>((gridDim.x * static_cast<int64_t>(blockDim.x)) >> 5);
+    for (int32_t i = p0 + warp; i < p1; i += n_warps) {
+        const uint32_t v = row_at[i];
+        const int32_t r = static_cast<int32_t>(v & 0x7fffffffu);
+        if (r >= n_rows) continue;
+        const bool absent = v >> 31;
+        uint8_t *row = e + static_cast<int64_t>(i - p0) * n_pad;
+        for (int32_t q = lane; q < n_pad / 16; q += 32) {
+            uint32_t fill[4] = {0u, 0u, 0u, 0u};                 // padding genomes (c >= N) stay 0
+            if (absent)
+                for (int b = 0; b < 16; ++b) fill[b >> 2] |= (16 * q + b < n ? 1u : 0u) << (8 * (b & 3));
+            reinterpret_cast<uint4 *>(row)[q] = make_uint4(fill[0], fill[1], fill[2], fill[3]);
+        }
+        __syncwarp();
+        for (int32_t x = sorted_ptr[r] + lane; x < sorted_ptr[r + 1]; x += 32) row[sorted_idx[x]] = absent ? 0 : 1;
+    }
+}
+
+// one block per 32 bitmap rows: those in the panel -> E rows, 4 genomes (one uint32 of bytes) per thread and row
+__global__ void __launch_bounds__(256) pair_expand_bitmap_kernel(const uint32_t *__restrict__ bits, int32_t n,
+                                                                 int32_t slice_words, int32_t n_long, int32_t n_rows,
+                                                                 const int32_t *__restrict__ pos_of, int32_t p0,
+                                                                 int32_t p1, int32_t n_pad, uint8_t *__restrict__ e)
+{
+    __shared__ int32_t dst[32];
+    const int32_t line = 32 * slice_words;
+    const int32_t sb = blockIdx.x / line, w = blockIdx.x % line;
+    bool mine = false;
+    if (threadIdx.x < 32) {
+        const int64_t k = static_cast<int64_t>(sb) * 1024 * slice_words + 32 * w + threadIdx.x;
+        const int32_t p = k < n_long ? pos_of[n_rows + k] : -1;
+        mine = p >= p0 && p < p1;
+        dst[threadIdx.x] = mine ? p - p0 : -1;
+    }
+    if (!__syncthreads_or(mine)) return;
+    for (int32_t q = threadIdx.x; q < n_pad / 4; q += blockDim.x) {
+        uint32_t v[4];
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            const int32_t c = 4 * q + j;
+            v[j] = c < n ? __ldg(&bits[(static_cast<int64_t>(sb) * n + c) * line + w]) : 0u;
+        }
+#pragma unroll 4
+        for (int b = 0; b < 32; ++b) {
+            const int32_t d = dst[b];
+            if (d < 0) continue;
+            const uint32_t out = ((v[0] >> b) & 1u) | ((v[1] >> b) & 1u) << 8 | ((v[2] >> b) & 1u) << 16 |
+                                 ((v[3] >> b) & 1u) << 24;
+            reinterpret_cast<uint32_t *>(e + static_cast<int64_t>(d) * n_pad)[q] = out;
+        }
+    }
+}
+
+// Histogram epilogue.  Buffer row i is sorted row base_lo + i below ``split`` and base_hi + i - split from it on.
+// A diagonal panel (split = buffer rows) counts the pairs i < j, a panel pair (split = P) the pairs i < split <= j.
+// Each tile's s and a lie in ranges known from the m of its first and last rows (rows sorted by m); when both fit
+// the stage buffers as uint32 bins they are counted there (at most BM x BN pairs: no bin can overflow) and added
+// into the global bins once, otherwise every pair goes straight to the global bins.
+constexpr int32_t PAIR_BINS = (STAGES * STAGE_BYTES - BN * 4) / 4;
+
+struct PairHistEpilogue {
+    const int32_t *m_sorted;
+    unsigned long long *hs, *ha;
+    int32_t n_stored, n, base_lo, base_hi, split;
+    bool cross;
+
+    __device__ __forceinline__ int32_t sorted_row(int32_t i) const
+    {
+        return i < split ? base_lo + i : base_hi + (i - split);
+    }
+
+    __device__ __forceinline__ bool skip(int32_t rb, int32_t cb) const
+    {
+        if (cross && (rb * BM >= split || (cb + 1) * BN <= split)) return true;
+        return sorted_row(rb * BM) >= n_stored || sorted_row(cb * BN) >= n_stored;
+    }
+
+    template <bool LOCAL>
+    __device__ __forceinline__ void count(uint32_t tmem, int warp, int lane, int32_t m0, int32_t n0,
+                                          const int32_t *col_m, uint32_t *bins, int32_t s_lo, int32_t sw,
+                                          int32_t a_lo) const
+    {
+        const int32_t row = m0 + 32 * warp + lane;
+        const int32_t gr = sorted_row(row);
+        const bool row_ok = gr < n_stored;
+        const int32_t base = n - (row_ok ? m_sorted[gr] : 0);
+#pragma unroll 1
+        for (int c = 0; c < BN; c += 32) {
+            uint32_t acc[32];
+            tmem_ld_32(tmem + (static_cast<uint32_t>(32 * warp) << 16) + c, acc);
+            if (!row_ok || (!cross && n0 + c + 31 <= row)) continue;
+#pragma unroll
+            for (int q = 0; q < 32; ++q) {
+                const int32_t mc = col_m[c + q];
+                if (mc < 0 || (!cross && n0 + c + q <= row)) continue;
+                const int32_t s = static_cast<int32_t>(acc[q]), a = base - mc + s;
+                if (LOCAL) {
+                    atomicAdd(bins + (s - s_lo), 1u);
+                    atomicAdd(bins + sw + (a - a_lo), 1u);
+                } else {
+                    atomicAdd(hs + s, 1ull);
+                    atomicAdd(ha + a, 1ull);
+                }
+            }
+        }
+    }
+
+    __device__ __forceinline__ void run(uint32_t tmem, int warp, int lane, int32_t m0, int32_t n0, int32_t,
+                                        uint32_t stages) const
+    {
+        extern __shared__ uint8_t smem_raw[];
+        int32_t *col_m = reinterpret_cast<int32_t *>(smem_raw + (stages - smem_u32(smem_raw)));
+        uint32_t *bins = reinterpret_cast<uint32_t *>(col_m + BN);
+        for (int j = threadIdx.x; j < BN; j += GEMM_THREADS) {
+            const int32_t g = sorted_row(n0 + j);
+            col_m[j] = g < n_stored ? m_sorted[g] : -1;
+        }
+        const int32_t r_lo = m_sorted[sorted_row(m0)], r_hi = m_sorted[min(sorted_row(m0 + BM - 1), n_stored - 1)];
+        const int32_t c_lo = m_sorted[sorted_row(n0)], c_hi = m_sorted[min(sorted_row(n0 + BN - 1), n_stored - 1)];
+        const int32_t s_lo = max(0, r_lo + c_lo - n), s_hi = min(r_hi, c_hi);
+        const int32_t a_lo = max(0, n - r_hi - c_hi), a_hi = n - max(r_lo, c_lo);
+        const int32_t sw = s_hi - s_lo + 1, width = sw + a_hi - a_lo + 1;
+        const bool local = width <= PAIR_BINS;
+        if (local)
+            for (int32_t v = threadIdx.x; v < width; v += GEMM_THREADS) bins[v] = 0;
+        __syncthreads();
+        if (local) {
+            count<true>(tmem, warp, lane, m0, n0, col_m, bins, s_lo, sw, a_lo);
+            __syncthreads();
+            for (int32_t v = threadIdx.x; v < width; v += GEMM_THREADS) {
+                const uint32_t x = bins[v];
+                if (x) atomicAdd(v < sw ? hs + s_lo + v : ha + a_lo + (v - sw), static_cast<unsigned long long>(x));
+            }
+        } else {
+            count<false>(tmem, warp, lane, m0, n0, col_m, bins, s_lo, sw, a_lo);
+        }
+    }
+};
+
+__global__ void __launch_bounds__(GEMM_THREADS, 1) pair_hist_gemm_kernel(const __grid_constant__ CUtensorMap map,
+                                                                          int32_t rows, int32_t k_blocks,
+                                                                          PairHistEpilogue epi)
+{
+    gemm_tiles(map, rows, k_blocks, epi);
+}
+
+// Double-double arithmetic (a value is hi + lo, |lo| <= ulp(hi) / 2): the pan variance Z + 2 T_a - Z^2 cancels two
+// terms of about Z^2 (4e10 at C4 for k = 1), so rho and the sums carry about 32 significant digits.
+struct dd {
+    double hi, lo;
+};
+
+__device__ __forceinline__ dd dd_norm(double s, double e)
+{
+    const double hi = s + e;
+    return {hi, e - (hi - s)};
+}
+
+__device__ __forceinline__ dd dd_add(dd x, dd y)
+{
+    const double s = x.hi + y.hi, b = s - x.hi;
+    const double e = (x.hi - (s - b)) + (y.hi - b) + x.lo + y.lo;
+    return dd_norm(s, e);
+}
+
+__device__ __forceinline__ dd dd_mul(dd x, dd y)
+{
+    const double p = x.hi * y.hi;
+    return dd_norm(p, fma(x.hi, y.hi, -p) + (x.hi * y.lo + x.lo * y.hi));
+}
+
+// (v - k) / v to double-double: the quotient and the exact remainder's quotient
+__device__ __forceinline__ dd dd_ratio(int32_t v, int32_t k)
+{
+    const double num = v - k, den = v, q = num / den;
+    return {q, fma(-q, den, num) / den};
+}
+
+__device__ __forceinline__ dd dd_shfl_up(dd x, int d)
+{
+    return {__shfl_up_sync(0xffffffffu, x.hi, d), __shfl_up_sync(0xffffffffu, x.lo, d)};
+}
+
+__device__ __forceinline__ dd dd_shfl_down(dd x, int d)
+{
+    return {__shfl_down_sync(0xffffffffu, x.hi, d), __shfl_down_sync(0xffffffffu, x.lo, d)};
+}
+
+// One warp per k: T_w[k] = sum over v = N .. k of w[v] rho(v, k), rho(N, k) = 1, rho(v - 1, k) = rho(v, k) (v - k) / v.
+// Lane j takes the j-th run of ``c`` values of v from the top; a multiplicative scan of the runs' products gives each
+// lane its starting rho; the lanes' sums are then added in a fixed tree, so two calls give the same bits.
+constexpr int MOMENT_WARPS = 4;
+
+__global__ void __launch_bounds__(32 * MOMENT_WARPS) rarefaction_moments_kernel(
+    const int64_t *__restrict__ spectrum, const int64_t *__restrict__ hs, const int64_t *__restrict__ ha,
+    int64_t n_genes, int32_t n, double *__restrict__ out)
+{
+    const int lane = threadIdx.x & 31;
+    const int32_t k = blockIdx.x * MOMENT_WARPS + (threadIdx.x >> 5) + 1;
+    if (k > n) return;
+    const int32_t len = n - k + 1, c = (len + 31) / 32;
+    const int32_t top = n - lane * c, bottom = max(k, top - c + 1);        // this lane: v = top .. bottom
+    dd run = {1.0, 0.0};
+    for (int32_t v = top; v >= bottom && v > k; --v) run = dd_mul(run, dd_ratio(v, k));
+    if (top < k) run = {1.0, 0.0};
+    // exclusive product scan over the lanes: rho(top, k) = product of the runs above this lane
+    dd rho = dd_shfl_up(run, 1);
+    if (lane == 0) rho = {1.0, 0.0};
+    for (int d = 1; d < 32; d <<= 1) {
+        const dd other = dd_shfl_up(rho, d);
+        if (lane >= d) rho = dd_mul(rho, other);
+    }
+    dd core = {0.0, 0.0}, none = {0.0, 0.0}, ts = {0.0, 0.0}, ta = {0.0, 0.0};
+    for (int32_t v = top; v >= bottom && rho.hi != 0.0; --v) {
+        core = dd_add(core, dd_mul(rho, dd{static_cast<double>(spectrum[v]), 0.0}));
+        none = dd_add(none, dd_mul(rho, dd{static_cast<double>(spectrum[n - v]), 0.0}));
+        if (hs) {
+            ts = dd_add(ts, dd_mul(rho, dd{static_cast<double>(hs[v]), 0.0}));
+            ta = dd_add(ta, dd_mul(rho, dd{static_cast<double>(ha[v]), 0.0}));
+        }
+        rho = dd_mul(rho, dd_ratio(v, k));
+    }
+    for (int d = 16; d > 0; d >>= 1) {
+        core = dd_add(core, dd_shfl_down(core, d));
+        none = dd_add(none, dd_shfl_down(none, d));
+        ts = dd_add(ts, dd_shfl_down(ts, d));
+        ta = dd_add(ta, dd_shfl_down(ta, d));
+    }
+    if (lane != 0) return;
+    const int64_t nn = n;
+    const dd g = {static_cast<double>(n_genes), 0.0};
+    const dd pan = dd_add(g, dd{-none.hi, -none.lo});
+    out[k - 1] = pan.hi + pan.lo;
+    out[2 * nn + k - 1] = core.hi + core.lo;
+    if (hs) {
+        const dd two = {2.0, 0.0};
+        const dd vp = dd_add(dd_add(none, dd_mul(two, ta)), dd_mul(dd{-none.hi, -none.lo}, none));
+        const dd vc = dd_add(dd_add(core, dd_mul(two, ts)), dd_mul(dd{-core.hi, -core.lo}, core));
+        out[nn + k - 1] = vp.hi + vp.lo;
+        out[3 * nn + k - 1] = vc.hi + vc.lo;
+    }
+}
+
 // ---- host -------------------------------------------------------------------------------------------------------
 PFN_cuTensorMapEncodeTiled_v12000 tensor_map_encoder()
 {
@@ -399,6 +965,116 @@ PFN_cuTensorMapEncodeTiled_v12000 tensor_map_encoder()
 int launch_blocks(int64_t work, int threads)
 {
     return static_cast<int>(std::max<int64_t>(1, std::min<int64_t>((work + threads - 1) / threads, 148 * 16)));
+}
+
+// ---- host: pair histograms ----------------------------------------------------------------------------------------
+int64_t align256(int64_t x)
+{
+    return (x + 255) / 256 * 256;
+}
+
+int32_t padded_genomes(int32_t n)
+{
+    return (n + BK - 1) / BK * BK;
+}
+
+// workspace of pgx_pair_overlap_histograms: the fixed part, then the E panels
+struct PairLayout {
+    int64_t cc, m_row, rows_m, wp_m, wa_m, cursor, row_at, m_sorted, pos_of, e;
+
+    PairLayout(int32_t n, int64_t rows)
+    {
+        cc = 0;
+        m_row = align256(sizeof(ClassCounts));
+        rows_m = m_row + align256(4 * rows);
+        wp_m = rows_m + align256(8 * (int64_t(n) + 1));
+        wa_m = wp_m + align256(8 * (int64_t(n) + 1));
+        cursor = wa_m + align256(8 * (int64_t(n) + 1));
+        row_at = cursor + align256(4 * (int64_t(n) + 1));
+        m_sorted = row_at + align256(4 * rows);
+        pos_of = m_sorted + align256(4 * rows);
+        e = pos_of + align256(4 * rows);
+    }
+};
+
+// E rows the workspace must hold: all stored rows (one panel), or at least two panels of 256 rows
+int64_t pair_min_e_rows(int64_t rows)
+{
+    return std::min<int64_t>((rows + BM - 1) / BM * BM, 2 * BN);
+}
+
+int check_pair_plan(const char *who, const pgx_plan *plan)
+{
+    const int32_t n = plan->n_genomes;
+    if (n < 1 || n > MAX_GENOMES) return pgx::fail(PGX_ERR_INVALID, "%s: n_genomes = %d outside 1 .. %d", who, n, MAX_GENOMES);
+    if (plan->n_genes < 0) return pgx::fail(PGX_ERR_INVALID, "%s: negative n_genes", who);
+    if (!plan->d_colsum || !plan->d_w_present || !plan->d_w_absent)
+        return pgx::fail(PGX_ERR_INVALID, "%s: plan without its per-genome vectors", who);
+    if (plan->n_rows < 0 || plan->n_tasks < 0 || plan->n_long < 0 || plan->n_superblocks < 0)
+        return pgx::fail(PGX_ERR_INVALID, "%s: negative plan sizes", who);
+    if (plan->n_rows > 0 && (!plan->d_tasks || !plan->d_sorted_idx || !plan->d_sorted_ptr))
+        return pgx::fail(PGX_ERR_INVALID, "%s: plan without its list rows", who);
+    if (plan->n_long > 0 && (!plan->d_bits || (plan->slice_words != 1 && plan->slice_words != 2 && plan->slice_words != 4) ||
+                             int64_t(plan->n_superblocks) * 1024 * plan->slice_words < plan->n_long))
+        return pgx::fail(PGX_ERR_INVALID, "%s: plan without a valid bitmap", who);
+    return PGX_OK;
+}
+
+// m (and with wp_m, Wp and Wa) of every list and bitmap row, counted by m
+int count_rows(const pgx_plan *plan, const ClassCounts *cc, uint32_t *m_row, unsigned long long *rows_m,
+               unsigned long long *wp_m, unsigned long long *wa_m, cudaStream_t s)
+{
+    const int32_t n = plan->n_genomes;
+    if (plan->n_tasks > 0) {
+        pair_list_rows_kernel<<<launch_blocks(int64_t(plan->n_tasks) * 32, 256), 256, 0, s>>>(
+            plan->d_tasks, plan->n_tasks, plan->d_sorted_idx, plan->d_sorted_ptr, plan->d_w_present, plan->d_w_absent,
+            n, cc, m_row, rows_m, wp_m, wa_m);
+        PGX_LAUNCH_CHECK("pair_list_rows_kernel");
+    }
+    if (plan->n_long > 0) {
+        pair_bitmap_rows_kernel<<<plan->n_superblocks * 32 * plan->slice_words, 256, 0, s>>>(
+            plan->d_bits, n, plan->slice_words, plan->n_long, plan->n_rows, plan->d_w_present, plan->d_w_absent, m_row,
+            rows_m, wp_m, wa_m);
+        PGX_LAUNCH_CHECK("pair_bitmap_rows_kernel");
+    }
+    return PGX_OK;
+}
+
+// sorted rows lo .. lo + rows - 1 -> E rows 0 .. rows - 1 at ``e``
+int expand_panel(const pgx_plan *plan, const uint32_t *row_at, const int32_t *pos_of, int32_t lo, int32_t rows,
+                 int32_t n_pad, uint8_t *e, cudaStream_t s)
+{
+    if (plan->n_rows > 0) {
+        pair_expand_list_kernel<<<launch_blocks(int64_t(rows) * 32, 256), 256, 0, s>>>(
+            row_at, lo, lo + rows, plan->n_rows, plan->d_sorted_idx, plan->d_sorted_ptr, plan->n_genomes, n_pad, e);
+        PGX_LAUNCH_CHECK("pair_expand_list_kernel");
+    }
+    if (plan->n_long > 0) {
+        pair_expand_bitmap_kernel<<<plan->n_superblocks * 32 * plan->slice_words, 256, 0, s>>>(
+            plan->d_bits, plan->n_genomes, plan->slice_words, plan->n_long, plan->n_rows, pos_of, lo, lo + rows, n_pad, e);
+        PGX_LAUNCH_CHECK("pair_expand_bitmap_kernel");
+    }
+    return PGX_OK;
+}
+
+// histogram GEMM over the first ``rows`` rows of E (tensor map over exactly those rows)
+int pair_gemm(uint8_t *e, int32_t rows, int32_t n_pad, const PairHistEpilogue &epi, cudaStream_t s)
+{
+    CUtensorMap map;
+    const cuuint64_t dims[2] = {static_cast<cuuint64_t>(n_pad), static_cast<cuuint64_t>(rows)};
+    const cuuint64_t strides[1] = {static_cast<cuuint64_t>(n_pad)};
+    const cuuint32_t box[2] = {BK, BM}, elem[2] = {1, 1};
+    const CUresult rc = tensor_map_encoder()(&map, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, e, dims, strides, box, elem,
+                                             CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
+                                             CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    if (rc != CUDA_SUCCESS)
+        return pgx::fail(PGX_ERR_CUDA, "pgx_pair_overlap_histograms: cuTensorMapEncodeTiled failed (%d)", int(rc));
+    const int32_t row_tiles = (rows + BM - 1) / BM, col_tiles = (rows + BN - 1) / BN;
+    int64_t tiles = 0;
+    for (int32_t g = 0; g * GROUP_ROWS < row_tiles; ++g) tiles += group_tiles(g, col_tiles);
+    pair_hist_gemm_kernel<<<static_cast<unsigned>(tiles), GEMM_THREADS, GEMM_SMEM, s>>>(map, rows, n_pad / BK, epi);
+    PGX_LAUNCH_CHECK("pair_hist_gemm_kernel");
+    return PGX_OK;
 }
 
 }  // namespace
@@ -504,6 +1180,141 @@ int pgx_fluidity_rows(const int32_t *d_shared, int32_t n_genomes, double *d_row_
     fluidity_rows_kernel<<<(n_genomes + ROWS - 1) / ROWS, ROW_THREADS, 0, static_cast<cudaStream_t>(stream)>>>(
         d_shared, n_genomes, d_row_sums);
     PGX_LAUNCH_CHECK("fluidity_rows_kernel");
+    return PGX_OK;
+}
+
+int64_t pgx_pair_overlap_work_bytes(int32_t n_genomes, int64_t n_stored_rows, int32_t one_panel)
+{
+    if (n_genomes < 1 || n_genomes > MAX_GENOMES || n_stored_rows < 0 || n_stored_rows > INT32_MAX - 2 * BN) return 0;
+    const int64_t e_rows = one_panel ? (n_stored_rows + BM - 1) / BM * BM : pair_min_e_rows(n_stored_rows);
+    return PairLayout(n_genomes, n_stored_rows).e + e_rows * padded_genomes(n_genomes);
+}
+
+int pgx_plan_spectrum(const pgx_plan *plan, int64_t *d_spectrum, void *stream)
+{
+    if (!plan || !d_spectrum) return pgx::fail(PGX_ERR_INVALID, "pgx_plan_spectrum: null pointer");
+    if ((reinterpret_cast<uintptr_t>(d_spectrum) & 7) != 0)
+        return pgx::fail(PGX_ERR_INVALID, "pgx_plan_spectrum: d_spectrum must be 8-byte aligned");
+    if (const int rc = check_pair_plan("pgx_plan_spectrum", plan)) return rc;
+    const int32_t n = plan->n_genomes;
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    PGX_CUDA(cudaMemsetAsync(d_spectrum, 0, sizeof(int64_t) * (size_t(n) + 1), s));
+    if (const int rc = count_rows(plan, nullptr, nullptr, reinterpret_cast<unsigned long long *>(d_spectrum), nullptr,
+                                  nullptr, s))
+        return rc;
+    spectrum_finish_kernel<<<1, 1024, 0, s>>>(n, plan->n_genes, int64_t(plan->n_rows) + plan->n_long, plan->d_colsum,
+                                             plan->d_w_present, plan->d_w_absent, d_spectrum);
+    PGX_LAUNCH_CHECK("spectrum_finish_kernel");
+    int64_t empty = 0;
+    PGX_CUDA(cudaMemcpyAsync(&empty, d_spectrum, sizeof(empty), cudaMemcpyDeviceToHost, s));
+    PGX_CUDA(cudaStreamSynchronize(s));
+    if (empty < 0)
+        return pgx::fail(PGX_ERR_INVALID, "pgx_plan_spectrum: inconsistent plan (rows and vectors do not add up to the "
+                                          "column sums in whole universal and empty genes)");
+    return PGX_OK;
+}
+
+int pgx_pair_overlap_histograms(const pgx_plan *plan, int64_t *d_hist_shared, int64_t *d_hist_absent, void *d_work,
+                                int64_t work_bytes, void *stream)
+{
+    if (!plan || !d_hist_shared || !d_hist_absent || !d_work)
+        return pgx::fail(PGX_ERR_INVALID, "pgx_pair_overlap_histograms: null pointer");
+    if ((reinterpret_cast<uintptr_t>(d_hist_shared) & 7) != 0 || (reinterpret_cast<uintptr_t>(d_hist_absent) & 7) != 0 ||
+        (reinterpret_cast<uintptr_t>(d_work) & 255) != 0)
+        return pgx::fail(PGX_ERR_INVALID, "pgx_pair_overlap_histograms: the histograms must be 8-byte and d_work "
+                                          "256-byte aligned");
+    if (const int rc = check_pair_plan("pgx_pair_overlap_histograms", plan)) return rc;
+    const int32_t n = plan->n_genomes, n_pad = padded_genomes(n);
+    const int64_t stored = int64_t(plan->n_rows) + plan->n_long;
+    const int64_t need = pgx_pair_overlap_work_bytes(n, stored, 0);
+    if (need == 0) return pgx::fail(PGX_ERR_INVALID, "pgx_pair_overlap_histograms: %lld stored rows", (long long)stored);
+    if (work_bytes < need)
+        return pgx::fail(PGX_ERR_INVALID, "pgx_pair_overlap_histograms: work_bytes = %lld below the minimum %lld",
+                         static_cast<long long>(work_bytes), static_cast<long long>(need));
+    if (stored > 1 && !tensor_map_encoder())
+        return pgx::fail(PGX_ERR_CUDA, "pgx_pair_overlap_histograms: the driver does not provide cuTensorMapEncodeTiled");
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    const PairLayout L(n, stored);
+    uint8_t *w = static_cast<uint8_t *>(d_work);
+    ClassCounts *cc = reinterpret_cast<ClassCounts *>(w + L.cc);
+    uint32_t *m_row = reinterpret_cast<uint32_t *>(w + L.m_row);
+    auto *rows_m = reinterpret_cast<unsigned long long *>(w + L.rows_m);
+    auto *wp_m = reinterpret_cast<unsigned long long *>(w + L.wp_m);
+    auto *wa_m = reinterpret_cast<unsigned long long *>(w + L.wa_m);
+    int32_t *cursor = reinterpret_cast<int32_t *>(w + L.cursor);
+    uint32_t *row_at = reinterpret_cast<uint32_t *>(w + L.row_at);
+    int32_t *m_sorted = reinterpret_cast<int32_t *>(w + L.m_sorted);
+    int32_t *pos_of = reinterpret_cast<int32_t *>(w + L.pos_of);
+    uint8_t *e = w + L.e;
+    auto *hs = reinterpret_cast<unsigned long long *>(d_hist_shared);
+    auto *ha = reinterpret_cast<unsigned long long *>(d_hist_absent);
+
+    PGX_CUDA(cudaMemsetAsync(w, 0, L.m_row, s));
+    PGX_CUDA(cudaMemsetAsync(w + L.rows_m, 0, L.cursor - L.rows_m, s));
+    PGX_CUDA(cudaMemsetAsync(hs, 0, sizeof(int64_t) * (size_t(n) + 1), s));
+    PGX_CUDA(cudaMemsetAsync(ha, 0, sizeof(int64_t) * (size_t(n) + 1), s));
+    pair_vectors_kernel<<<1, 1024, 0, s>>>(n, plan->d_colsum, plan->d_w_present, plan->d_w_absent, cc);
+    PGX_LAUNCH_CHECK("pair_vectors_kernel");
+    if (const int rc = count_rows(plan, cc, m_row, rows_m, wp_m, wa_m, s)) return rc;
+    pair_classes_kernel<<<1, 1024, 0, s>>>(n, plan->n_genes, stored, rows_m, cc);
+    PGX_LAUNCH_CHECK("pair_classes_kernel");
+    // a plan whose rows and vectors do not add up to its column sums would give wrong histograms: refuse it before
+    // the heavy phases (the only point at which the call waits for the device)
+    ClassCounts host{};
+    PGX_CUDA(cudaMemcpyAsync(&host, cc, sizeof(host), cudaMemcpyDeviceToHost, s));
+    PGX_CUDA(cudaStreamSynchronize(s));
+    if (!host.valid)
+        return pgx::fail(PGX_ERR_INVALID, "pgx_pair_overlap_histograms: inconsistent plan (rows and vectors do not add "
+                                          "up to the column sums in whole universal and empty genes)");
+    pair_closed_kernel<<<(n + 1 + 255) / 256, 256, 0, s>>>(n, cc, rows_m, wp_m, wa_m, hs, ha);
+    PGX_LAUNCH_CHECK("pair_closed_kernel");
+    if (stored < 2) return PGX_OK;
+
+    pair_scan_kernel<<<1, 1024, 0, s>>>(n, rows_m, cursor);
+    PGX_LAUNCH_CHECK("pair_scan_kernel");
+    pair_sort_kernel<<<static_cast<unsigned>((stored + 255) / 256), 256, 0, s>>>(static_cast<int32_t>(stored), m_row,
+                                                                                 cursor, row_at, m_sorted, pos_of);
+    PGX_LAUNCH_CHECK("pair_sort_kernel");
+
+    // one panel when every stored row fits, else panels of P rows (a multiple of BN), two at a time
+    const int64_t e_rows = (work_bytes - L.e) / n_pad;
+    const int32_t panel = e_rows >= (stored + BM - 1) / BM * BM ? static_cast<int32_t>(stored)
+                                                                 : static_cast<int32_t>(e_rows / 2 / BN * BN);
+    PGX_CUDA(cudaFuncSetAttribute(pair_hist_gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM));
+    PairHistEpilogue epi{m_sorted, hs, ha, static_cast<int32_t>(stored), n, 0, 0, 0, false};
+    for (int32_t lo_i = 0; lo_i < stored; lo_i += panel) {
+        const int32_t rows_i = static_cast<int32_t>(std::min<int64_t>(panel, stored - lo_i));
+        if (const int rc = expand_panel(plan, row_at, pos_of, lo_i, rows_i, n_pad, e, s)) return rc;
+        epi.base_lo = lo_i, epi.base_hi = static_cast<int32_t>(stored), epi.split = rows_i, epi.cross = false;
+        if (const int rc = pair_gemm(e, rows_i, n_pad, epi, s)) return rc;
+        for (int32_t lo_j = lo_i + panel; lo_j < stored; lo_j += panel) {
+            const int32_t rows_j = static_cast<int32_t>(std::min<int64_t>(panel, stored - lo_j));
+            if (const int rc = expand_panel(plan, row_at, pos_of, lo_j, rows_j, n_pad, e + int64_t(panel) * n_pad, s))
+                return rc;
+            epi.base_hi = lo_j, epi.split = panel, epi.cross = true;
+            if (const int rc = pair_gemm(e, panel + rows_j, n_pad, epi, s)) return rc;
+        }
+    }
+    return PGX_OK;
+}
+
+int pgx_rarefaction_moments(const int64_t *d_spectrum, const int64_t *d_hist_shared, const int64_t *d_hist_absent,
+                            int64_t n_genes, int32_t n_genomes, double *d_out, void *stream)
+{
+    if (!d_spectrum || !d_out) return pgx::fail(PGX_ERR_INVALID, "pgx_rarefaction_moments: null pointer");
+    if (!d_hist_shared != !d_hist_absent)
+        return pgx::fail(PGX_ERR_INVALID, "pgx_rarefaction_moments: pass both histograms or neither");
+    if (n_genomes < 1 || n_genomes > MAX_GENOMES)
+        return pgx::fail(PGX_ERR_INVALID, "pgx_rarefaction_moments: n_genomes = %d outside 1 .. %d", n_genomes,
+                         MAX_GENOMES);
+    if (n_genes < 0) return pgx::fail(PGX_ERR_INVALID, "pgx_rarefaction_moments: negative n_genes");
+    if (((reinterpret_cast<uintptr_t>(d_spectrum) | reinterpret_cast<uintptr_t>(d_hist_shared) |
+          reinterpret_cast<uintptr_t>(d_hist_absent) | reinterpret_cast<uintptr_t>(d_out)) & 7) != 0)
+        return pgx::fail(PGX_ERR_INVALID, "pgx_rarefaction_moments: every pointer must be 8-byte aligned");
+    rarefaction_moments_kernel<<<(n_genomes + MOMENT_WARPS - 1) / MOMENT_WARPS, 32 * MOMENT_WARPS, 0,
+                                 static_cast<cudaStream_t>(stream)>>>(
+        d_spectrum, d_hist_shared, d_hist_absent, n_genes, n_genomes, d_out);
+    PGX_LAUNCH_CHECK("rarefaction_moments_kernel");
     return PGX_OK;
 }
 

@@ -332,8 +332,62 @@ class PanCoreEngine:
                                                      torch.cuda.current_stream(self.device).cuda_stream))
         return rows
 
+    # ---- exact rarefaction over all genome orders -------------------------------------------------------------
+    def spectrum_device(self):
+        """Gene-frequency spectrum of the table from its plan (pgx_plan_spectrum): a CUDA int64 tensor [N + 1], entry
+        v = genes present in exactly v genomes.  Asynchronous on the current torch stream after a short wait in which
+        the library checks the plan."""
+        torch = _torch()
+        out = torch.empty(self.n_genomes + 1, dtype=torch.int64, device=self.device)
+        with torch.cuda.device(self.device):
+            _native.check(self.lib.pgx_plan_spectrum(ctypes.byref(self.c_plan), out.data_ptr(),
+                                                     torch.cuda.current_stream(self.device).cuda_stream))
+        return out
 
-SHARED_WORK_CAP = 4 << 30          # bytes of expanded bitmap rows per slab of pgx_shared_genes
+    def pair_workspace_bytes(self):
+        """Workspace of pgx_pair_overlap_histograms: every stored row's E row in one panel, at most SHARED_WORK_CAP
+        bytes of E rows (a larger table takes several panels), at least the minimum the call needs."""
+        hp, n = self.host_plan, self.n_genomes
+        stored = hp.n_rows + hp.n_long
+        least = int(self.lib.pgx_pair_overlap_work_bytes(n, stored, 0))
+        whole = int(self.lib.pgx_pair_overlap_work_bytes(n, stored, 1))
+        fixed = whole - -(-stored // 128) * 128 * (-(-n // 128) * 128)
+        return max(least, min(whole, fixed + SHARED_WORK_CAP))
+
+    def pair_histograms_device(self, work_bytes=None):
+        """Pair overlap histograms (pgx_pair_overlap_histograms) as two CUDA int64 tensors [N + 1]: H_s[v] = gene pairs
+        g < h present together in exactly v genomes, H_a[v] = pairs absent together from exactly v genomes.  The
+        workspace (pair_workspace_bytes() unless given) is a torch allocation, released on return.  Asynchronous on
+        the current torch stream after a short wait in which the library checks the plan."""
+        torch = _torch()
+        n = self.n_genomes
+        hs = torch.empty(n + 1, dtype=torch.int64, device=self.device)
+        ha = torch.empty(n + 1, dtype=torch.int64, device=self.device)
+        work_bytes = int(work_bytes or self.pair_workspace_bytes())
+        with torch.cuda.device(self.device):
+            work = torch.empty(work_bytes, dtype=torch.uint8, device=self.device)
+            _native.check(self.lib.pgx_pair_overlap_histograms(
+                ctypes.byref(self.c_plan), hs.data_ptr(), ha.data_ptr(), work.data_ptr(), work_bytes,
+                torch.cuda.current_stream(self.device).cuda_stream))
+        return hs, ha
+
+    def exact_moments_device(self, std=True):
+        """Mean and variance of the pan and core curves over all genome orders (pgx_rarefaction_moments) as a CUDA
+        float64 tensor [4, N]: rows E[pan_k], Var[pan_k], E[core_k], Var[core_k], k = 1 .. N.  With std=False no pair
+        histograms are computed, no workspace is allocated and the variance rows are NaN."""
+        torch = _torch()
+        n = self.n_genomes
+        spectrum = self.spectrum_device()
+        hs, ha = self.pair_histograms_device() if std else (None, None)
+        out = torch.full((4, n), float("nan"), dtype=torch.float64, device=self.device)
+        with torch.cuda.device(self.device):
+            _native.check(self.lib.pgx_rarefaction_moments(
+                spectrum.data_ptr(), hs.data_ptr() if std else None, ha.data_ptr() if std else None, self.n_genes, n,
+                out.data_ptr(), torch.cuda.current_stream(self.device).cuda_stream))
+        return out
+
+
+SHARED_WORK_CAP = 4 << 30          # bytes of expanded rows per slab / panel of pgx_shared_genes and the pair histograms
 
 
 def fit_heaps_device(curves, n_points=None):

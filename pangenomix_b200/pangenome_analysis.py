@@ -14,7 +14,9 @@ reference; the work is done by libpgx_b200 on a B200:
 
 Extension beside the drop-in: ``estimate_pan_core_summary`` -- mean / std / min / max of the pan/core curves over
 genome orders drawn on the GPU from a seeded counter-based stream (not numpy's), reduced on the GPU;
-``shared_gene_counts`` (genome x genome shared genes, X^T X on the tensor cores) and ``compute_genomic_fluidity``.
+``shared_gene_counts`` (genome x genome shared genes, X^T X on the tensor cores) and ``compute_genomic_fluidity``;
+``exact_pan_core_summary`` -- the exact mean and std of the pan/core curves over ALL genome orders, without sampling
+(gene-pair overlap histograms counted on the tensor cores).
 
 Not provided (out of scope, SURVEY.md section 2): the coordinate-descent variant the
 reference marks "DON'T USE THIS" and the mlst wrapper.
@@ -197,6 +199,42 @@ def estimate_pan_core_summary(df_genes, num_iter, seed=0, device=None):
     _, num_strains = df_genes.shape
     engine = _engine_for(df_genes, device)
     return summary_frame(engine.summary(num_iter, seed), num_strains)
+
+
+def exact_pan_core_summary(df_genes, std=True, device=None):
+    '''
+    Exact mean and standard deviation of the pan/core curves over ALL orders of the genomes, without sampling: the
+    quantities estimate_pan_core_summary() estimates.  The first k genomes of a random order are a random k-subset,
+    so with rho(v, k) = C(v, k) / C(N, k), E[core_k] = sum over genes of rho(m_g, k) and E[pan_k] = G - sum over genes
+    of rho(N - m_g, k) (Mao's tau, Colwell, Mao & Chang 2004).  The variances add the pairs of genes: how many genomes
+    each pair shares and how many lack both, counted on the GPU from the table's plan (shared with
+    estimate_pan_core_size / estimate_pan_core_summary), the dense part as an 8-bit integer matrix product on the
+    tensor cores.  The result is deterministic: no seed, no sampling noise.  Prints nothing and leaves ``np.random``
+    untouched.
+
+    Parameters
+    ----------
+    df_genes : LightSparseDataFrame
+        Sparse binary gene x genome table (anything with .shape and a scipy .data)
+    std : bool
+        Also compute the std (default).  False computes the means only, which need just the gene-frequency spectrum.
+    device : optional CUDA device (default: current device)
+
+    Returns
+    -------
+    df_stats : pd.DataFrame
+        float64, index ['mean', 'std'] (['mean'] with std=False), columns Pan1..PanN, Core1..CoreN.  ``std`` is the
+        exact standard deviation over the orders of these N genomes, sqrt(max(Var, 0)); exactly 0 at k = N.
+        ``df_stats.loc[['mean']]`` can be passed to fit_heaps_by_iteration() / fit_heaps_by_iteration_gpu().
+    '''
+    _, num_strains = df_genes.shape
+    engine = _engine_for(df_genes, device)
+    moments = engine.exact_moments_device(std=std).cpu().numpy()
+    rows = [np.concatenate([moments[0], moments[2]])]
+    if std:
+        rows.append(np.sqrt(np.maximum(np.concatenate([moments[1], moments[3]]), 0.0)))
+    return pd.DataFrame(np.vstack(rows), index=['mean', 'std'] if std else ['mean'],
+                        columns=_labels(('Pan', 'Core'), num_strains), copy=False)
 
 
 def summary_frame(moments, num_strains):
